@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the per-marker quantification hot path (BASELINE.json metric: ROI-pixels/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c1..c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config c1..c5] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Default workload (config.workload): BASELINE config 3, "chip time series" -- per rank 50
@@ -412,6 +412,11 @@ def run_b200_arm(args, name, cfg):
     barrier()
     launches = lib.mgb_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        outputs = {"image": image_out}
+        if has_markers:
+            outputs.update(roi=roi_out, stats=symm.gathered[rank] if symm is not None else stats_out)
+        dump_outputs(args.dump_outputs, outputs)
     elapsed_s = max_over_ranks(start.elapsed_time(end)) / 1e3
     value = unit_px_rank * world * args.steps / elapsed_s
 
@@ -517,6 +522,35 @@ def run_b200_arm(args, name, cfg):
         dist.barrier(group=group)
         dist.destroy_process_group()
     return line
+
+
+DUMP_MAX_ELEMENTS = 1 << 20
+
+
+def dump_outputs(directory, outputs):
+    """Write the arrays of the last timed step as DIR/<name>.npy (uint16 -> float32, float64 kept)
+    so that two builds can be compared output for output.  An array of more than
+    DUMP_MAX_ELEMENTS elements is replaced by a sample at fixed, seeded flat (C-order) positions,
+    written beside it as DIR/<name>_index.npy (float64); every file together stays under 64 MB."""
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    for seed, (name, tensor) in enumerate(outputs.items()):
+        dtype = np.float64 if tensor.dtype == torch.float64 else np.float32
+        # CUDA indexing has no uint16 kernel: gather the same bits as int16 and reinterpret on the host
+        unsigned16 = tensor.dtype == torch.uint16
+        src = tensor.view(torch.int16) if unsigned16 else tensor
+        n = tensor.numel()
+        if n <= DUMP_MAX_ELEMENTS:
+            values = src.cpu().numpy()
+        else:
+            index = np.unique(np.random.default_rng(seed).integers(0, n, DUMP_MAX_ELEMENTS, dtype=np.int64))
+            coords = tuple(torch.from_numpy(a).to(tensor.device) for a in np.unravel_index(index, tuple(tensor.shape)))
+            values = src[coords].cpu().numpy()
+            np.save(os.path.join(directory, f"{name}_index.npy"), index.astype(np.float64))
+        if unsigned16:
+            values = values.view(np.uint16)
+        np.save(os.path.join(directory, f"{name}.npy"), values.astype(dtype))
 
 
 def sampled_parity(case, plan, image, roi, stats, group=None):
@@ -916,7 +950,14 @@ def main():
                     help="N>1: gather the summaries with NCCL all_gather instead of peer stores from the kernel")
     ap.add_argument("--config", default="c3", choices=sorted(CONFIGS),
                     help="c3 = BASELINE config 3 (default, the metric's workload); c1, c2, c4, c5 = the other configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the image, crops and summaries of the last step as DIR/<name>.npy "
+                         "(large arrays as a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     cfg = dict(CONFIGS[args.config])
     if args.timepoints:
         cfg["t"] = args.timepoints

@@ -12,113 +12,18 @@ needed (and does not exist) on the GPU box; centres are pinned to the ones the r
 tests/test_dropin_reference.py is the other half: the same layer inside the reference's real
 Pipeline, on the CPU stand-in for the kernels.
 """
-import json
-import os
-
-import numpy as np
 import pytest
 
+from dropin_cases import replay_bead_case, replay_chip_case
+
 pytestmark = pytest.mark.gpu
-
-GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
-
-def load_state(g, prefix):
-    from magnify_b200.dataset import Dataset
-
-    data, coords = {}, {}
-    for entry in g[prefix + "__names"]:
-        kind, name = str(entry).split(":", 1)
-        dims = tuple(str(d) for d in g[f"{prefix}__{name}__dims"])
-        (coords if kind == "coord" else data)[name] = (dims, g[f"{prefix}__{name}"])
-    return Dataset(data, coords)
-
-
-class Registry(dict):
-    def register(self, name):
-        return lambda f: self.__setitem__(name, f) or f
-
-    def get(self, name):
-        return self[name]
-
-
-def run_pipe(components, assay):
-    for _, component in components:          # pipeline.py:19-22
-        assay = component(assay)
-    return assay
-
-
-def compare(got, want, names):
-    for name in names:
-        a, b = got[name], want[name]
-        assert tuple(a.dims) == tuple(b.dims), (name, a.dims, b.dims)
-        av, bv = np.asarray(a.values), np.asarray(b.values)
-        assert av.dtype == bv.dtype and av.shape == bv.shape, (name, av.dtype, bv.dtype, av.shape, bv.shape)
-        np.testing.assert_array_equal(av, bv, err_msg=name)
-        assert (name in got.coords) == (name in want.coords), name
 
 
 @pytest.mark.parametrize("case", ["chip_single", "chip_series", "chip_tiles", "chip_blank_float"])
 def test_chip_components_reproduce_reference_pipeline(cuda_device, case):
-    from magnify_b200 import components
-    from magnify_b200.devarray import DeviceArray
-
-    g = np.load(os.path.join(GOLDEN, f"dropin_{case}.npz"))
-    kw = json.loads(str(g["kwargs_json"]))
-    assay, want = load_state(g, "in"), load_state(g, "out")
-    rows, cols = want["tag"].shape if want["tag"].ndim == 2 else (None, None)
-    search = sorted(np.atleast_1d(kw["search_timestep"]).tolist())
-    wx = np.asarray(want["x"].values)
-    wy = np.asarray(want["y"].values)
-    m = wx.shape[0]
-    grid = (int(np.asarray(want["mark_row"].values).max()) + 1, int(np.asarray(want["mark_col"].values).max()) + 1)
-
-    def centers(xp, t):
-        k = search.index(t)
-        return wx[:, t].reshape(grid), wy[:, t].reshape(grid), g["fg_radius"][k].reshape(grid)
-
-    reg = Registry()
-    components.install(registry=reg)
-    finder_kw = {k: kw[k] for k in ("row_dist", "col_dist", "min_button_diameter", "max_button_diameter", "chamber_diameter",
-                                    "top_chamber", "left_chamber", "low_edge_quantile", "high_edge_quantile", "num_iter",
-                                    "min_roundness", "cluster_penalty", "roi_length", "progress_bar", "search_timestep",
-                                    "search_channel", "interactive")}
-    pipe = [("stitch", reg.get("stitch")(overlap=kw["overlap"])),
-            ("find_buttons", reg.get("find_buttons")(**finder_kw, centers=centers))]
-    got = run_pipe(pipe, assay)
-    assert isinstance(got["image"].data, DeviceArray) and isinstance(got["roi"].data, DeviceArray)   # nothing left the GPU yet
-    assert got["roi"].shape[0] == m
-    compare(got, want, ["image", "roi", "fg", "bg", "x", "y", "valid", "tag", "mark_row", "mark_col"])
-    # and the summaries of the same pass equal the xarray expressions on the reference's dataset
-    got = reg.get("quantify")()(got)
-    if np.asarray(want["roi"].values).dtype == np.uint16:
-        sel = want["roi"].where(want["fg"])
-        np.testing.assert_array_equal(got["fg_median"].values, sel.median(dim=["roi_x", "roi_y"]).values)
-        np.testing.assert_allclose(got["fg_mean"].values, sel.mean(dim=["roi_x", "roi_y"]).values, rtol=1e-6)
-    # the consumers of the crops, in the order the golden generator ran the reference's own
-    # (filter.py:11-94): medians and contour perimeters from the kernels, `valid` must follow exactly
-    for name, fkw in (("filter_expression", {}), ("filter_nonround", {"min_roundness": 0.6}), ("filter_leaky", {})):
-        got = reg.get(name)(**fkw)(got)
-        np.testing.assert_array_equal(np.asarray(got["valid"].values), g[f"valid_after__{name}"], err_msg=name)
+    replay_chip_case(case)
 
 
 @pytest.mark.parametrize("case", ["beads_single", "beads_flatfield_tiles", "beads_none"])
 def test_bead_components_reproduce_reference_pipeline(cuda_device, case):
-    from magnify_b200 import components
-
-    g = np.load(os.path.join(GOLDEN, f"dropin_{case}.npz"))
-    kw = json.loads(str(g["kwargs_json"]))
-    assay, want = load_state(g, "in"), load_state(g, "out")
-    beads = g["beads"]                       # the centres and radii the reference's (pinned) search returned
-    reg = Registry()
-    components.install(registry=reg)
-    finder_kw = {k: kw[k] for k in ("min_bead_diameter", "max_bead_diameter", "low_edge_quantile", "high_edge_quantile",
-                                    "num_iter", "min_roundness", "roi_length", "search_channel", "interactive")}
-    pipe = []
-    flat = g["kwarg__flatfield"] if "kwarg__flatfield" in g else kw["flatfield"]
-    dark = g["kwarg__darkfield"] if "kwarg__darkfield" in g else kw["darkfield"]
-    pipe.append(("flatfield_correct", reg.get("flatfield_correct")(flatfield=flat, darkfield=dark)))
-    pipe.append(("stitch", reg.get("stitch")(overlap=kw["overlap"])))
-    pipe.append(("find_beads", reg.get("find_beads")(**finder_kw, centers=beads)))
-    got = run_pipe(pipe, assay)
-    compare(got, want, ["image", "roi", "fg", "bg", "x", "y", "valid"])
+    replay_bead_case(case)

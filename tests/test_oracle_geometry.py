@@ -1,6 +1,6 @@
 """The oracle's integer geometry against the golden vectors made from the reference's real
-utils.py (tests/golden/make_golden.py), against cv2, and -- when /root/reference is present --
-against the reference itself."""
+utils.py (tests/golden/make_golden.py and make_reference_record.py), against cv2, and -- when
+the reference is present -- against the reference itself."""
 import numpy as np
 import pytest
 
@@ -64,19 +64,50 @@ def test_cv_circle_against_cv2():
             np.testing.assert_array_equal(g.circle((72, 72), (cy, cx), r), img.astype(bool))
 
 
-def test_against_reference_utils_when_present():
-    u = load_reference_utils()
-    if u is None:
-        pytest.skip("/root/reference not available (GPU box); goldens cover this")
+GEOMETRY_RADII = (1, 2, 3, 7, 16, 33, 100, 257)
+
+
+def geometry_cases():
     rng = np.random.default_rng(0)
+    boxes = []
     for _ in range(3000):
         w, h, length = rng.integers(1, 300, 3)
         x, y = rng.integers(-50, 350, 2)
-        assert tuple(int(v) for v in u.bounding_box(int(x), int(y), int(length), int(w), int(h))) == \
-            g.bounding_box(int(x), int(y), int(length), int(w), int(h))
-    for r in (1, 2, 3, 7, 16, 33, 100, 257):
-        assert np.array_equal(u.circle_points(r), g.circle_points(r))
-        assert np.array_equal(u.circle_points(r, True), g.circle_points(r, True))
-        assert set(map(tuple, u.filled_circle_points(r).tolist())) == set(map(tuple, g.filled_circle_points(r).tolist()))
+        boxes.append((int(x), int(y), int(length), int(w), int(h)))
     beads = np.stack([rng.integers(-5, 150, 40), rng.integers(-5, 170, 40), rng.integers(1, 20, 40)], 1)
-    np.testing.assert_array_equal(u.circle_labels(beads, 140, 160), g.circle_labels(beads, 140, 160))
+    return boxes, beads
+
+
+def sorted_points(points):
+    return np.array(sorted(map(tuple, np.asarray(points).tolist())))
+
+
+def record():
+    """This package's side of every comparison with the reference in this module (written to
+    tests/golden/reference_record.npz by tests/golden/make_reference_record.py)."""
+    boxes, beads = geometry_cases()
+    out = {"bounding_boxes": np.array([g.bounding_box(*args) for args in boxes]),
+           "circle_labels": g.circle_labels(beads, 140, 160)}
+    for r in GEOMETRY_RADII:
+        out[f"circle_points_{r}"], out[f"circle_points4_{r}"] = g.circle_points(r), g.circle_points(r, True)
+        out[f"filled_circle_points_{r}"] = sorted_points(g.filled_circle_points(r))
+    return out
+
+
+def test_against_reference_utils_when_present(golden):
+    """What the reference's utils.py returned (tests/golden/reference_record.npz), and the
+    reference itself when it is present."""
+    rec, u = golden("reference_record"), load_reference_utils()
+    boxes, beads = geometry_cases()
+    for args, want in zip(boxes, rec["bounding_boxes"]):
+        assert g.bounding_box(*args) == tuple(int(v) for v in want)
+        if u is not None:
+            assert tuple(int(v) for v in u.bounding_box(*args)) == tuple(int(v) for v in want)
+    sides = [g] if u is None else [g, u]
+    for r in GEOMETRY_RADII:
+        for side in sides:
+            np.testing.assert_array_equal(side.circle_points(r), rec[f"circle_points_{r}"])
+            np.testing.assert_array_equal(side.circle_points(r, True), rec[f"circle_points4_{r}"])
+            np.testing.assert_array_equal(sorted_points(side.filled_circle_points(r)), rec[f"filled_circle_points_{r}"])
+    for side in sides:
+        np.testing.assert_array_equal(side.circle_labels(beads, 140, 160), rec["circle_labels"])

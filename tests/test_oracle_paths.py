@@ -56,16 +56,42 @@ def test_stitch_golden_from_reference_source(golden):
         np.testing.assert_array_equal(got, g[name + "__image"], err_msg=name)
 
 
-def test_stitch_against_reference_source_when_present():
+STITCH_OVERLAPS = (0, 1, 4, 7, 13)
+
+
+def stitch_tiles():
+    return np.random.default_rng(3).integers(0, 65535, (2, 2, 3, 2, 14, 18), dtype=np.uint16, endpoint=True)
+
+
+def flatfield_case():
+    rng = np.random.default_rng(7)
+    tiles = rng.integers(0, 65535, (2, 1, 2, 2, 16, 16), dtype=np.uint16, endpoint=True)
+    flat = 0.6 + 0.8 * rng.random((16, 16))
+    dark = 80 + 40 * rng.random((16, 16))
+    return tiles, flat, dark
+
+
+def record():
+    """This package's side of the stitch and flat-field comparisons with the reference in this
+    module (written to tests/golden/reference_record.npz by tests/golden/make_reference_record.py)."""
+    tiles = stitch_tiles()
+    out = {f"stitch_{ov}": st.stitch(tiles, ov) for ov in STITCH_OVERLAPS}
+    out["flatfield"] = ff.flatfield_correct(*flatfield_case())
+    return out
+
+
+def test_stitch_against_reference_source_when_present(golden):
+    """What the reference's Stitcher returned (tests/golden/reference_record.npz), and the
+    reference itself when it is present."""
     from oracle._refload import reference_stitch
 
-    rng = np.random.default_rng(3)
-    tiles = rng.integers(0, 65535, (2, 2, 3, 2, 14, 18), dtype=np.uint16, endpoint=True)
-    for ov in (0, 1, 4, 7, 13):
-        want = reference_stitch(tiles, ov)
-        if want is None:
-            pytest.skip("/root/reference not available (GPU box); the golden fixture covers this")
+    rec, tiles = golden("reference_record"), stitch_tiles()
+    for ov in STITCH_OVERLAPS:
+        want = rec[f"stitch_{ov}"]
         np.testing.assert_array_equal(st.stitch(tiles, ov), want)
+        ref = reference_stitch(tiles, ov)
+        if ref is not None:
+            np.testing.assert_array_equal(ref, want)
 
 
 # ---- flat-field ------------------------------------------------------------------------------
@@ -113,17 +139,16 @@ def test_flatfield_golden_from_reference_source(golden):
     np.testing.assert_array_equal(got, g["f32__out"])
 
 
-def test_flatfield_against_reference_source_when_present():
+def test_flatfield_against_reference_source_when_present(golden):
+    """What the reference's flatfield_correct returned (tests/golden/reference_record.npz), and
+    the reference itself when it is present."""
     from oracle._refload import reference_flatfield_correct
 
-    rng = np.random.default_rng(7)
-    tiles = rng.integers(0, 65535, (2, 1, 2, 2, 16, 16), dtype=np.uint16, endpoint=True)
-    flat = 0.6 + 0.8 * rng.random((16, 16))
-    dark = 80 + 40 * rng.random((16, 16))
-    want = reference_flatfield_correct(tiles, flat, dark)
-    if want is None:
-        pytest.skip("/root/reference not available (GPU box); the golden fixture covers this")
-    np.testing.assert_array_equal(ff.flatfield_correct(tiles, flat, dark), want)
+    want = golden("reference_record")["flatfield"]
+    np.testing.assert_array_equal(ff.flatfield_correct(*flatfield_case()), want)
+    ref = reference_flatfield_correct(*flatfield_case())
+    if ref is not None:
+        np.testing.assert_array_equal(ref, want)
 
 
 # ---- ROI paths against fixtures made with the reference's real utils.py -----------------------
@@ -193,15 +218,19 @@ def test_chip_multi_search_golden(golden, make_pattern_image):
 def test_finders_against_reference_source_when_present(golden, make_pattern_image):
     """The committed bead / chip fixtures equal what the reference's own BeadFinder /
     ButtonFinder `__call__` (find.py, executed in place with the stochastic centre finder
-    pinned) produce on the same inputs."""
+    pinned) produce on the same inputs; without the reference, what the oracle's masks and crops
+    produce from the same centres."""
     from oracle._refload import reference_bead_finder, reference_button_finder
 
     d = golden("beads")
     c, t, h, w = (int(v) for v in d["image_shape"])
     image = make_pattern_image(c, t, h, w, salt=int(d["image_salt"]))
     ref = reference_bead_finder(image, ["a", "b"], d["beads"], int(d["roi_length"]))
-    if ref is None:
-        pytest.skip("/root/reference not available (GPU box); the golden fixtures cover this")
+    if ref is None:   # without the reference: the oracle's restatement of the finders against the same fixtures
+        labels, fg, bg = rois.bead_masks(d["beads"], h, w, int(d["roi_length"]))
+        x, y = np.repeat(d["beads"][:, 1:2], t, 1), np.repeat(d["beads"][:, 0:1], t, 1)
+        ref = {"roi": rois.gather_rois(image, x, y, int(d["roi_length"])), "fg": np.repeat(fg[:, None], t, 1),
+               "bg": np.repeat(bg[:, None], t, 1)}
     np.testing.assert_array_equal(ref["roi"], d["roi"])
     for ti in range(t):
         np.testing.assert_array_equal(ref["fg"][:, ti], d["fg"])
@@ -213,6 +242,12 @@ def test_finders_against_reference_source_when_present(golden, make_pattern_imag
     rows, cols = d["x"].shape
     refine = [None if r[2] < 0 else tuple(int(v) for v in r) for r in d["refine"].reshape(-1, 3)]
     ref = reference_button_finder(image, ["a", "b"], np.full((rows, cols), "default"), d["coarse_x"], d["coarse_y"], refine)
+    if ref is None:
+        x, y, length = d["x"].reshape(-1), d["y"].reshape(-1), int(d["roi_length"])
+        fg, bg = rois.chip_masks(x, y, d["fg_radius"].reshape(-1), length, int(d["chamber_radius"]),
+                                 int(d["max_button_radius"]), w, h)
+        ref = {"roi": rois.gather_rois(image, np.repeat(x[:, None], t, 1), np.repeat(y[:, None], t, 1), length),
+               "fg": np.repeat(fg[:, None], t, 1), "bg": np.repeat(bg[:, None], t, 1), "x": x[:, None]}
     np.testing.assert_array_equal(ref["roi"], d["roi"])
     np.testing.assert_array_equal(ref["fg"], d["fg"])
     np.testing.assert_array_equal(ref["bg"], d["bg"])
@@ -266,15 +301,18 @@ def test_filter_expression_golden_from_reference_source(golden):
 
 
 def test_filter_expression_against_reference_source_when_present(golden):
+    """filter.npz against the reference's own filter_expression, with xarray's `where` promoting
+    to the input type and to float64; without the reference, the oracle against the same golden."""
     from oracle._refload import reference_filter_expression
 
     g = golden("filter")
     for names, search, mc, want in filter_cases(g):
+        idx = list(range(len(names))) if search is None else [names.index(s) for s in search]
+        np.testing.assert_array_equal(red.filter_expression_valid(g["roi"], g["fg"], g["bg"], g["valid"], idx, mc), want)
         for promote in (None, np.float64):
             got = reference_filter_expression(g["roi"], g["fg"], g["bg"], g["valid"], names, search, mc, promote)
-            if got is None:
-                pytest.skip("/root/reference not available (GPU box); the golden fixture covers this")
-            np.testing.assert_array_equal(got, want)
+            if got is not None:
+                np.testing.assert_array_equal(got, want)
 
 
 def test_mrbles_intensities_golden_from_reference_expression(golden):

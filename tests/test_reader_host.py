@@ -150,15 +150,36 @@ def test_extract_paths_contract(tmp_path):
         reader.extract_paths(patterns(str(tmp_path))[5], **KEYS)
 
 
-def test_extract_paths_against_reference_source_when_present(tmp_path):
+def canonical_outcome(fn, root):
+    """repr of each pattern's outcome with its mappings in sorted order and the tree's root
+    written as <root>."""
+    def canonical(result):
+        if isinstance(result, str):
+            return result
+        paths, meta = result
+        return (sorted(paths.items(), key=repr), sorted(((k, sorted(v.items(), key=repr)) for k, v in meta.items()), key=repr))
+
+    return [repr(canonical(outcome(fn, pattern))).replace(root, "<root>") for pattern in patterns(root)]
+
+
+def record(tmpdir):
+    """This package's side of the comparison with the reference's extract_paths (written to
+    tests/golden/reference_record.npz by tests/golden/make_reference_record.py)."""
+    make_tree(tmpdir)
+    return {"extract_paths": np.array(canonical_outcome(reader.extract_paths, tmpdir))}
+
+
+def test_extract_paths_against_reference_source_when_present(tmp_path, golden):
+    """What the reference's extract_paths returned (tests/golden/reference_record.npz), and the
+    reference itself when it is present."""
     from oracle._refload import load_reference_reader
 
-    ref = load_reference_reader()
-    if ref is None:
-        pytest.skip("/root/reference not available (GPU box)")
+    want = [str(v) for v in golden("reference_record")["extract_paths"]]
     make_tree(str(tmp_path))
-    for pattern in patterns(str(tmp_path)):
-        assert outcome(reader.extract_paths, pattern) == outcome(ref.extract_paths, pattern), pattern
+    assert canonical_outcome(reader.extract_paths, str(tmp_path)) == want
+    ref = load_reference_reader()
+    if ref is not None:
+        assert canonical_outcome(ref.extract_paths, str(tmp_path)) == want
 
 
 # ---- tile stack assembly ---------------------------------------------------------------------
