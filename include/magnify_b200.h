@@ -159,7 +159,7 @@ int mgb_roi_gather(const void* image, int64_t image_pitch, int64_t C, int64_t T,
  * search timestep, find.py:151,172-173); any non-zero mask byte counts as set.  roi may be NULL
  * (summaries only).  stats (M,C,T,8) float64: counts, exact integer sums, mean = sum / count (NaN
  * for an empty mask, like nanmean), and the exact masked medians (mean of the two middle values
- * for even counts, NaN for an empty mask, like nanmedian).
+ * for even counts, NaN for an empty mask, like nanmedian).  stats must be 16-byte aligned.
  *
  * fg_count_max / bg_count_max: upper bounds of the number of set pixels in any fg / bg mask (from
  * mgb_mask_count_max, or -1 = unknown).  With bounds of at most 1024 / 2560 pixels the kernel
@@ -181,7 +181,8 @@ int mgb_mask_count_max(const uint8_t* fg, const uint8_t* bg, int64_t n_masks, in
  * EVERY rank over NVLink peer memory (no separate all-gather).  host_peer_stats[j] (host array of
  * n_peers <= 8 device addresses) points at THIS rank's (M,C,T,8) block inside rank j's gathered
  * (ranks,M,C,T,8) buffer (peer-mapped, e.g. torch symmetric memory); the caller synchronises the
- * ranks afterwards.  Needs the staged kernels (else MGB_EUNSUPPORTED). */
+ * ranks afterwards.  Every peer address must be 16-byte aligned.  Needs the staged kernels (else
+ * MGB_EUNSUPPORTED). */
 int mgb_roi_gather_stats_peers_u16(const uint16_t* image, int64_t image_pitch, int64_t C, int64_t T,
                                    int64_t H, int64_t W, const int32_t* boxes, const int32_t* order, const int32_t* mask_t,
                                    int64_t Tm, const uint8_t* fg, const uint8_t* bg, int64_t M, int L,

@@ -481,7 +481,8 @@ static int gather_common(const void* image, int64_t image_pitch, int64_t C, int6
   if (n_peers > 0) return MGB_EUNSUPPORTED;   // peer write-out exists only in the staged kernels
   const int unit = itemsize / 2;
   const int Lu = L * (unit ? unit : 1);
-  const bool word_path = itemsize >= 2 && (Lu % 2 == 0) &&
+  // (Lu > 2: a row of one word has no 32-bit multiply-high magic number for its division)
+  const bool word_path = itemsize >= 2 && (Lu % 2 == 0) && Lu > 2 &&
                          ((reinterpret_cast<uintptr_t>(image) & 3u) == 0) &&
                          (!roi || (reinterpret_cast<uintptr_t>(roi) & 3u) == 0) &&
                          (!with_stats || ((reinterpret_cast<uintptr_t>(fg) & 1u) == 0 &&

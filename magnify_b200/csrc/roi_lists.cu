@@ -541,14 +541,16 @@ int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int
   const bool out8 = !roi || (reinterpret_cast<uintptr_t>(roi) & 7u) == 0;
   const bool out4 = !roi || (reinterpret_cast<uintptr_t>(roi) & 3u) == 0;
   int vpl = 0, qpl = 0;
-  if (wu % 8 == 0 && out16) {
+  // the copy loops divide by vpr / half with a multiply-high by ceil(2^32 / d), which has no 32-bit
+  // value for d = 1: rows of one vector (L = 8) take the quads, rows of one word (L = 2) the generic loop
+  if (wu % 8 == 0 && wu > 8 && out16) {
     p.vpr = (uint32_t)(wu / 8);
     p.magic_vpr = magic_u32_(p.vpr);
     const int v = (int)((L * p.vpr + 31) / 32);
     vpl = v <= 12 ? 12 : v <= 21 ? 21 : v <= 36 ? 36 : 0;
   } else if (wu % 2 == 0 && (L * wu) % 4 == 0 && out8 && (L * wu / 4 + 31) / 32 <= 24) {
     qpl = (L * wu / 4 + 31) / 32 <= 12 ? 12 : 24;
-  } else if (wu % 2 == 0 && out4) {
+  } else if (wu % 2 == 0 && wu > 2 && out4) {
     p.half = (uint32_t)(wu / 2);
     p.magic_half = magic_u32_(p.half);
   }

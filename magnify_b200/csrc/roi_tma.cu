@@ -421,10 +421,12 @@ int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64
   p.stage_bytes = (L * wpu * 2 + 127) & ~127;
   const bool out16 = !roi || aligned16(roi);
   const bool out4 = !roi || (reinterpret_cast<uintptr_t>(roi) & 3u) == 0;
-  if (wu % 8 == 0 && out16) {
+  // vpr / half = 1 has no 32-bit multiply-high magic number (ceil(2^32 / 1)): rows of one vector take
+  // the word loop, rows of one word the generic loop
+  if (wu % 8 == 0 && wu > 8 && out16) {
     p.vpr = (uint32_t)(wu / 8);
     p.magic_vpr = magic_u32(p.vpr);
-  } else if (wu % 2 == 0 && out4) {
+  } else if (wu % 2 == 0 && wu > 2 && out4) {
     p.half = (uint32_t)(wu / 2);
     p.magic_half = magic_u32(p.half);
   }

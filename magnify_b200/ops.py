@@ -403,6 +403,8 @@ def roi_gather(image: torch.Tensor, boxes: torch.Tensor, roi_length: int, out: O
         out = torch.empty(shape, dtype=image.dtype, device=image.device)
     elif tuple(out.shape) != shape or out.dtype != image.dtype:
         raise ValueError(f"out must have shape {shape} and dtype {image.dtype}")
+    elif not out.is_contiguous():
+        raise ValueError("out must be contiguous")   # the kernels write roi + n*L*L densely
     with torch.cuda.device(image.device):
         _lib.call("mgb_roi_gather", _ptr(image), pitch, c, t, h, w, image.element_size(), _ptr(boxes),
                   _ptr(_check_order(order, m)), m, int(roi_length), _ptr(out), _stream())
@@ -496,6 +498,19 @@ def roi_gather_stats(
         roi = out_roi if out_roi is not None else torch.empty(shape, dtype=image.dtype, device=image.device)
         if tuple(roi.shape) != shape or roi.dtype != image.dtype:
             raise ValueError(f"out_roi must have shape {shape} and dtype {image.dtype}")
+        if not roi.is_contiguous():
+            raise ValueError("out_roi must be contiguous")   # the kernels write roi + n*L*L densely
+    # the staged kernels store each 64-byte summary record as four 16-byte vectors
+    if peer_stats is not None:
+        if any(int(a) % 16 for a in peer_stats):
+            raise ValueError("every peer_stats address must be 16-byte aligned")
+    else:
+        stats = out_stats if out_stats is not None else torch.empty((m, c, t, NSTATS), dtype=torch.float64,
+                                                                    device=image.device)
+        if tuple(stats.shape) != (m, c, t, NSTATS) or stats.dtype != torch.float64 or not stats.is_contiguous():
+            raise ValueError(f"out_stats must be contiguous float64 with shape (M, C, T, {NSTATS})")
+        if stats.data_ptr() % 16:
+            raise ValueError("out_stats must be 16-byte aligned")
     if mask_counts is None:
         mask_counts = mask_count_max(fg, bg) if m * tm > 0 else (0, 0)
     nf_max, nb_max = int(mask_counts[0]), int(mask_counts[1])
@@ -513,10 +528,6 @@ def roi_gather_stats(
             raise RuntimeError("peer_stats needs the fused gather (masks of at most 1024 fg / 2560 bg pixels per marker, "
                                "uint16 image); gather locally and all_gather the summaries instead")
         return roi, None
-    stats = out_stats if out_stats is not None else torch.empty((m, c, t, NSTATS), dtype=torch.float64,
-                                                                device=image.device)
-    if tuple(stats.shape) != (m, c, t, NSTATS) or stats.dtype != torch.float64 or not stats.is_contiguous():
-        raise ValueError(f"out_stats must be contiguous float64 with shape (M, C, T, {NSTATS})")
     with torch.cuda.device(image.device):
         _lib.call("mgb_roi_gather_stats_u16", _ptr(image), pitch, c, t, h, w, _ptr(boxes), _ptr(_check_order(order, m)),
                   _ptr(mask_t), tm, _ptr(fg), _ptr(bg), m, int(roi_length), _ptr(roi), _ptr(stats),

@@ -720,16 +720,24 @@ def test_gather_fused_medians(cuda_device, monkeypatch, layout, length, r_fg, r_
     assert np.isnan(no_med[..., 6:]).all()
 
 
+_SPLIT_TAILS = [(9, None, False)] + [(k, w, True) for k in (1, 9, "third", "last") for w in (6, 12)]
+
+
+@pytest.mark.parametrize("tail", _SPLIT_TAILS, ids=[f"k{k}-w{w or 'auto'}-{'perm' if o else 'id'}" for k, w, o in _SPLIT_TAILS])
 @pytest.mark.parametrize("c,t", [(3, 10), (4, 33)])
-def test_gather_split_last_wave(cuda_device, monkeypatch, c, t):
+def test_gather_split_last_wave(cuda_device, monkeypatch, c, t, tail):
     """A few more markers than a multiple of the resident CTAs: the markers of the last, nearly
     empty wave are shared by several CTAs each (roi_lists.cu).  Same crops and summaries as the
     oracle and as the unsplit launch, with few windows per marker (two 6-warp CTAs per SM) and
-    with many (one 12-warp CTA)."""
+    with many (one 12-warp CTA).  tail = (k, warps, order): M = 2 x SMs + k markers for k = 1, 9,
+    SMs / 3 ("third") and SMs - 1 ("last"), at 6 or 12 warps per CTA, with the markers in a random
+    processing order (the split deals marker slots, which `order` then maps to markers)."""
     from magnify_b200 import ops
 
     sms = torch.cuda.get_device_properties(cuda_device).multi_processor_count
-    m, length, h, w = 2 * sms + 9, 33, 200, 320
+    k, warps, shuffle = tail
+    k = {"third": sms // 3, "last": sms - 1}.get(k, k)
+    m, length, h, w = 2 * sms + k, 33, 200, 320
     rng = np.random.default_rng(c * 100 + t)
     image = np.clip(rng.normal(700, 60, (c, t, h, w)), 0, 65535).astype(np.uint16)
     x = rng.uniform(0, w, (m, t))
@@ -740,11 +748,18 @@ def test_gather_split_last_wave(cuda_device, monkeypatch, c, t):
     boxes = ops.bounding_boxes(dev(x, cuda_device), dev(y, cuda_device), length, w, h)
     fg_d, bg_d = dev(fg.view(np.uint8), cuda_device), dev(bg.view(np.uint8), cuda_device)
     counts = ops.mask_count_max(fg_d, bg_d)
+    order = dev(rng.permutation(m).astype(np.int32), cuda_device) if shuffle else None
     monkeypatch.setenv("MGB_GATHER_LAYOUT", "0")
+    if warps:
+        monkeypatch.setenv("MGB_GATHER_WARPS", str(warps))
+    else:
+        monkeypatch.delenv("MGB_GATHER_WARPS", raising=False)
     results = []
     for split in ("1", "0"):
         monkeypatch.setenv("MGB_GATHER_SPLIT", split)
-        roi, stats = ops.roi_gather_stats(dev(image, cuda_device), boxes, fg_d, bg_d, length, mask_counts=counts)
+        roi, stats = ops.roi_gather_stats(dev(image, cuda_device), boxes, fg_d, bg_d, length, mask_counts=counts,
+                                          order=order)
+        assert ops.last_gather_fused is True
         np.testing.assert_array_equal(roi.cpu().numpy(), want_roi)
         got = stats.cpu().numpy()
         np.testing.assert_array_equal(got[..., :4], want[..., :4])
