@@ -412,7 +412,7 @@ ff_apply_generic_kernel(const T* __restrict__ tiles, T* __restrict__ out, int64_
   }
 }
 
-static int g_stitch_variant = 0;   // tuning knob: 0 = 6 stages x 2 CTAs/SM, 1 = 10 x 2, 2 = 8 x 3
+static int g_stitch_variant = 0;   // tuning knob: 0 = 6 stages x 2 CTAs/SM, 1 = 11 x 2, 2 = 8 x 3
 
 template <int MODE, int D, int B>
 static int launch_stitch_variant(const StitchParams& p, cudaStream_t st) {
