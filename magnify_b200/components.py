@@ -26,6 +26,7 @@ from __future__ import annotations
 
 import math
 import os
+from dataclasses import dataclass
 from typing import Callable, Optional
 
 import numpy as np
@@ -127,36 +128,20 @@ def _stage_tiles(src, dev, ff: Optional[ops.FlatFieldPlan]) -> torch.Tensor:
     tiles = torch.empty(shape, dtype=dtype, device=dev)
     if tiles.numel() == 0:
         return tiles
-    compute = torch.cuda.current_stream(dev)
-    streams = devarray.Streams.of(dev)
-    streams.h2d.wait_stream(compute)
-    if maxima:
-        ff.maxima.zero_()
-
-    def landed(ci, ti, ev):
-        compute.wait_event(ev)
-        if maxima:
-            ops.flatfield_maxima_accumulate(tiles[ci, ti], ff, ci)
-
+    h2d = devarray.Streams.of(dev).h2d
     if isinstance(src, np.ndarray) and _is_pinned(src):
         host = torch.from_numpy(src)
-        for ti in range(shape[1]):
-            for ci in range(shape[0]):
-                with torch.cuda.stream(streams.h2d):
-                    tiles[ci, ti].copy_(host[ci, ti], non_blocking=True)
-                    ev = torch.cuda.Event()
-                    ev.record(streams.h2d)
-                landed(ci, ti, ev)
+        pipeline.upload_blocks((((ci, ti), host[ci, ti]) for ti in range(shape[1]) for ci in range(shape[0])), tiles,
+                               h2d, ff)
     else:
         # pageable memory, dask chunks, TIFF pages: through a ring of pinned slots
         blocks = src.blocks() if callable(getattr(src, "blocks", None)) else pipeline.iter_blocks(src)
         ring = pipeline.PinnedRing(shape[2:], dtype)
         try:
-            for (ci, ti), block in blocks:
-                landed(ci, ti, ring.send(block, tiles[ci, ti], streams.h2d))
+            pipeline.upload_blocks(blocks, tiles, h2d, ff, ring)
         finally:
             ring.close()
-    tiles.record_stream(streams.h2d)
+    tiles.record_stream(h2d)
     return tiles
 
 
@@ -260,6 +245,31 @@ def _channel_names(assay, n_channels: int):
     return list(_to_numpy(assay["channel"])) if "channel" in assay else list(range(n_channels))
 
 
+# ---------------------------------------------------------------------------------------------
+# marker boxes and masks (find.py:143-181, 380-400, 543-586), shared with pipeline.QuantifyPlan
+# ---------------------------------------------------------------------------------------------
+# host -> device uploads of the marker code: ops.upload_async, reached through this module so that a
+# test can replace it together with `ops`
+_upload = ops.upload_async
+
+
+@dataclass
+class Markers:
+    """Boxes and masks of M markers over T timepoints, built on the device from host arrays by
+    `chip_markers` / `bead_markers` for the finders and for `pipeline.QuantifyPlan`.  Every upload
+    is pinned and non-blocking and nothing is read back, so building them never waits behind
+    transfers already queued on the device."""
+    x: torch.Tensor                    # (M, T) float64 centres
+    y: torch.Tensor
+    boxes: torch.Tensor                # (M, T, 2) int32 (top, left)
+    fg: torch.Tensor                   # (M, Tm, L, L) uint8, one mask per mask timestep
+    bg: torch.Tensor
+    mask_t: torch.Tensor               # (T,) int32: the mask timestep of every timepoint
+    mask_t_host: np.ndarray            # the same as int64 (DeviceArray.take)
+    count_bounds: tuple                # upper bounds of the fg / bg pixel counts, from the radii
+    labels: Optional[torch.Tensor] = None   # beads: the (Him, Wim) int32 label raster
+
+
 def _disc_pixels(radius: int) -> int:
     """Pixels of {dx^2 + dy^2 <= r^2}: an upper bound of any disc mask of that radius inside a window."""
     r = int(radius)
@@ -267,33 +277,73 @@ def _disc_pixels(radius: int) -> int:
     return int((d[:, None] ** 2 + d[None, :] ** 2 <= r * r).sum())
 
 
-def _upload(values: np.ndarray, dev) -> torch.Tensor:
-    """Small host array -> device on the current stream WITHOUT blocking the host: a pageable copy
-    waits for everything queued on the stream (the tile upload and the stitch of this assay), which
-    would keep the next assay's upload from being queued behind this one's."""
-    host = torch.from_numpy(np.ascontiguousarray(values))
-    return host.pin_memory().to(dev, non_blocking=True)   # torch's caching host allocator holds the block until the copy ran
+def chip_markers(x, y, fg_radius, search_timesteps, chamber_radius: int, max_button_radius: int, roi_length: int,
+                 image_shape, device) -> Markers:
+    """Chip buttons (find.py:143-181, 380-400): x, y (M, T) float64 centres in image coordinates,
+    already copied forward; fg_radius (M, Ts) int, the refined radius or max_button_radius per
+    search timestep.  fg is the button disc, bg the annulus max_button_radius < d <= chamber_radius."""
+    x = np.asarray(x, dtype=np.float64)
+    y = np.asarray(y, dtype=np.float64)
+    if x.ndim != 2 or x.shape != y.shape:
+        raise ValueError("x and y must have shape (M, T)")
+    m, t = x.shape
+    src = pipeline.copy_forward_sources(t, search_timesteps)
+    search = sorted(set(src.tolist()))
+    fg_radius = np.asarray(fg_radius, dtype=np.int32).reshape(m, -1)
+    if fg_radius.shape[1] != len(search):
+        raise ValueError("fg_radius must have one column per search timestep")
+    him, wim = image_shape[-2:]
+    xd, yd = _upload(x, device), _upload(y, device)
+    boxes, rel = ops.bounding_boxes(xd, yd, roi_length, wim, him, want_rel=True)
+    masks = [ops.chip_masks(rel[:, ts].contiguous(), _upload(fg_radius[:, k], device), int(max_button_radius),
+                            int(chamber_radius), roi_length) for k, ts in enumerate(search)]
+    fg = torch.stack([f for f, _ in masks], 1).contiguous()
+    bg = torch.stack([b for _, b in masks], 1).contiguous()
+    mask_t = np.searchsorted(search, src).astype(np.int64)                              # find.py:172-173
+    bounds = (_disc_pixels(fg_radius.max()) if m else 0,
+              max(0, _disc_pixels(chamber_radius) - _disc_pixels(max_button_radius)))
+    return Markers(xd, yd, boxes, fg, bg, _upload(mask_t.astype(np.int32), device), mask_t, bounds)
 
 
-def _gather(image, boxes, fg, bg, mask_t, length, mask_counts):
-    """Crops of every marker, plus the summaries when the image dtype has the fused kernel.
-    mask_counts: host-side upper bounds of the fg / bg pixel counts (they size the kernel's value
-    lists).  Computed from the radii instead of read back from the device: a device->host read
-    here would queue behind the stitched image already on its way to the host and stall the
-    whole pipeline for the length of that transfer."""
-    if image.dtype == torch.uint16 and boxes.shape[0] > 0:
-        return ops.roi_gather_stats(image, boxes, fg, bg, length, mask_t=mask_t, medians=True, mask_counts=mask_counts)
-    return ops.roi_gather(image, boxes, length), None
+def bead_markers(beads, num_times: int, roi_length: int, image_shape, device) -> Markers:
+    """Beads (find.py:543-586): beads (M, 3) rows (row, col, radius), constant over time; fg / bg
+    from the label raster, one mask timestep for all timepoints."""
+    beads = np.asarray(beads, dtype=np.float64).reshape(-1, 3)
+    m, t = len(beads), int(num_times)
+    him, wim = image_shape[-2:]
+    xd = _upload(np.repeat(beads[:, 1:2], t, axis=1), device)
+    yd = _upload(np.repeat(beads[:, 0:1], t, axis=1), device)
+    boxes = ops.bounding_boxes(xd, yd, roi_length, wim, him)
+    labels = ops.bead_labels(beads.astype(np.int64).astype(np.int32), him, wim, device=device)   # astype(int), find.py:561
+    box0 = boxes[:, 0].contiguous() if t > 0 else torch.zeros((m, 2), dtype=torch.int32, device=device)
+    fg, bg = ops.bead_masks(labels, box0, roi_length)
+    # a bead's fg is at most its own disc (utils.py:398-430), its bg at most the whole window
+    rmax = max(int(beads[:, 2].max()), 1) if m else 1
+    hw = ops.disc_halfwidth_table(rmax)[rmax]
+    bounds = (int((2 * hw + 1).sum() * 2 - (2 * hw[0] + 1)), roi_length * roi_length)
+    return Markers(xd, yd, boxes, fg[:, None].contiguous(), bg[:, None].contiguous(),
+                   torch.zeros(t, dtype=torch.int32, device=device), np.zeros(t, dtype=np.int64), bounds, labels)
 
 
-def _emit_markers(roi_d, stats, fg_d, bg_d, mask_t: np.ndarray, mask_t_d):
+def _gather(image, mk: Markers, length):
+    """Crops of every marker, plus the summaries when the image dtype has the fused kernel.  The
+    gather's value lists are sized by the markers' count bounds, computed from the radii instead of
+    read back from the device: a device->host read here would queue behind the stitched image
+    already on its way to the host and stall the whole pipeline for the length of that transfer."""
+    if image.dtype == torch.uint16 and mk.boxes.shape[0] > 0:
+        return ops.roi_gather_stats(image, mk.boxes, mk.fg, mk.bg, length, mask_t=mk.mask_t, medians=True,
+                                    mask_counts=mk.count_bounds)
+    return ops.roi_gather(image, mk.boxes, length), None
+
+
+def _emit_markers(roi_d, stats, mk: Markers):
     """DeviceArrays of the crops and of the (M,T,L,L) masks.  The masks live on the device as their
     distinct timesteps (M,Tm,L,L) and expand lazily; later components find the compact tensors
     and the summaries the gather computed in `extras`."""
-    extras = {"stats": stats, "fg": fg_d, "bg": bg_d, "mask_t": mask_t_d}
+    extras = {"stats": stats, "fg": mk.fg, "bg": mk.bg, "mask_t": mk.mask_t}
     roi = _emit(roi_d, extras=extras, name="roi")
-    fg = _emit(fg_d, as_bool=True, extras=extras, prefetch=False).take(mask_t, 1)
-    bg = _emit(bg_d, as_bool=True, extras=extras, prefetch=False).take(mask_t, 1)
+    fg = _emit(mk.fg, as_bool=True, extras=extras, prefetch=False).take(mk.mask_t_host, 1)
+    bg = _emit(mk.bg, as_bool=True, extras=extras, prefetch=False).take(mk.mask_t_host, 1)
     return roi, fg, bg
 
 
@@ -351,7 +401,7 @@ class BeadFinder:
         dev = _device(self.device)
         image = _image_on_device(assay, dev)
         beads = self.find_centers(assay, image)
-        c, t, him, wim = image.shape
+        c, t = image.shape[:2]
         length = self.roi_length
         m = len(beads)
         x = np.repeat(beads[:, 1:2], t, axis=1)  # find.py:543-550
@@ -362,17 +412,8 @@ class BeadFinder:
             fg = np.empty((0, t, length, length), dtype=bool)
             bg = fg.copy()
         else:
-            boxes = ops.bounding_boxes(_upload(x, dev), _upload(y, dev), length, wim, him)
-            labels = ops.bead_labels(beads.astype(np.int64).astype(np.int32), him, wim, device=dev)
-            fg_d, bg_d = ops.bead_masks(labels, boxes[:, 0].contiguous(), length)
-            # masks are time invariant (find.py:585-586): one timestep on the device, broadcast on the host
-            fg_d, bg_d = fg_d[:, None].contiguous(), bg_d[:, None].contiguous()
-            mask_t_d = torch.zeros(t, dtype=torch.int32, device=dev)
-            # a bead's fg is at most its own disc (utils.py:398-430), its bg at most the whole window
-            hw = ops.disc_halfwidth_table(max(int(beads[:, 2].max()), 1))[max(int(beads[:, 2].max()), 1)]
-            counts = (int((2 * hw + 1).sum() * 2 - (2 * hw[0] + 1)), length * length)
-            roi_d, stats = _gather(image, boxes, fg_d, bg_d, mask_t_d, length, counts)
-            roi, fg, bg = _emit_markers(roi_d, stats, fg_d, bg_d, np.zeros(t, dtype=np.int64), mask_t_d)
+            mk = bead_markers(beads, t, length, image.shape, dev)
+            roi, fg, bg = _emit_markers(*_gather(image, mk, length), mk)
         assay["roi"] = (("mark", "channel", "time", "roi_y", "roi_x"), roi)
         return assay.assign_coords(
             fg=(("mark", "time", "roi_y", "roi_x"), fg), bg=(("mark", "time", "roi_y", "roi_x"), bg),
@@ -496,37 +537,18 @@ class ButtonFinder:
     def __call__(self, assay):
         dev = _device(self.device)
         image = _image_on_device(assay, dev)
-        c, t, him, wim = image.shape
+        c, t = image.shape[:2]
         rows, cols = assay["tag"].shape
-        m = rows * cols
         length = self.roi_length
-        src = pipeline.copy_forward_sources(t, self.search_timesteps)  # find.py:143-151
-        search = sorted(set(src.tolist()))
-        x = np.empty((rows, cols, t))
-        y = np.empty((rows, cols, t))
-        radius = np.empty((m, len(search)), dtype=np.int32)
-        for k, ts in enumerate(search):
-            xs, ys, rs = self.centers(assay, ts) if self.centers is not None else self._gpu_centers(assay, image, ts)
-            x[..., ts], y[..., ts], radius[:, k] = xs, ys, np.asarray(rs).reshape(m)
-        for ti in range(t):  # copy-forward of the centres, find.py:156-157,174-175
-            x[..., ti], y[..., ti] = x[..., src[ti]], y[..., src[ti]]
-        xd, yd = _upload(x.reshape(m, t), dev), _upload(y.reshape(m, t), dev)
-        boxes, rel = ops.bounding_boxes(xd, yd, length, wim, him, want_rel=True)
-        fgs, bgs = [], []
-        for k, ts in enumerate(search):
-            f, b = ops.chip_masks(rel[:, ts].contiguous(), _upload(radius[:, k], dev),
-                                  self.max_button_radius, self.chamber_radius, length)
-            fgs.append(f)
-            bgs.append(b)
-        fg_d, bg_d = torch.stack(fgs, 1).contiguous(), torch.stack(bgs, 1).contiguous()   # (M, Ts, L, L)
-        index = {ts: k for k, ts in enumerate(search)}
-        mask_t = np.array([index[int(s)] for s in src], dtype=np.int64)                   # find.py:172-173
-        mask_t_d = _upload(mask_t.astype(np.int32), dev)
-        counts = (_disc_pixels(int(radius.max())), max(0, _disc_pixels(self.chamber_radius) - _disc_pixels(self.max_button_radius)))
-        roi_d, stats = _gather(image, boxes, fg_d, bg_d, mask_t_d, length, counts)
+        find = self.centers if self.centers is not None else (lambda xp, ts: self._gpu_centers(xp, image, ts))
+        x, y, radius, src = pipeline.search_centers(lambda ts: find(assay, ts), t, self.search_timesteps)
+        mk = chip_markers(x, y, radius, self.search_timesteps, self.chamber_radius, self.max_button_radius, length,
+                                   image.shape, dev)
+        roi_d, stats = _gather(image, mk, length)
         valid = _to_numpy(assay["valid"]) if "valid" in assay else np.ones((rows, cols, t), dtype=bool)
         valid = valid[:, :, src] if valid.ndim == 3 else valid
-        roi, fg, bg = _emit_markers(roi_d, stats, fg_d, bg_d, mask_t, mask_t_d)
+        roi, fg, bg = _emit_markers(roi_d, stats, mk)
+        x, y = x.reshape(rows, cols, t), y.reshape(rows, cols, t)
         grid = ("mark_row", "mark_col")
         # the reference's layout before its stack (find.py:89-116), then its own stack + transpose (find.py:182)
         assay["roi"] = (grid + ("channel", "time", "roi_y", "roi_x"), roi.reshape(rows, cols, c, t, length, length))

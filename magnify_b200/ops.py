@@ -297,9 +297,9 @@ def flatfield_stitch(
         if maxima is None:
             maxima = flatfield_maxima(tiles, plan)
             if group is not None:
-                import torch.distributed as dist
+                from .dist import allreduce_maxima
 
-                dist.all_reduce(maxima, op=dist.ReduceOp.MAX, group=group)
+                allreduce_maxima(maxima, group)
         else:
             _check(maxima, "maxima", dtype=torch.float64)
             if maxima.data_ptr() != plan.maxima.data_ptr():
@@ -633,9 +633,11 @@ def disc_halfwidth_table(rmax: int) -> np.ndarray:
     return table
 
 
-def _upload_async(values: np.ndarray, device) -> torch.Tensor:
+def upload_async(values: np.ndarray, device) -> torch.Tensor:
     """Host array -> device on the current stream without blocking the host (pinned staging from
-    torch's caching host allocator, which keeps the block until the copy has run)."""
+    torch's caching host allocator, which keeps the block until the copy has run).  A pageable
+    copy would wait for everything already queued on the stream, such as an assay's tile upload
+    and stitch, and keep the next assay's work from being queued behind it."""
     return torch.from_numpy(np.ascontiguousarray(values)).pin_memory().to(device, non_blocking=True)
 
 
@@ -654,7 +656,7 @@ def bead_labels(beads, im_y: int, im_x: int, device=None) -> torch.Tensor:
             raise ValueError("beads must be (M,3)")
         m = host.shape[0]
         rmin, rmax = (int(host[:, 2].min()), int(host[:, 2].max())) if m else (1, 0)
-        beads = _upload_async(host, torch.device(device))
+        beads = upload_async(host, torch.device(device))
     else:
         _check(beads, "beads", dtype=torch.int32, ndim=2)
         m = beads.shape[0]
@@ -664,7 +666,7 @@ def bead_labels(beads, im_y: int, im_x: int, device=None) -> torch.Tensor:
     if m and rmin < 1:
         raise ValueError("bead radii must be >= 1 (filled_circle_points(0) raises in the reference)")
     labels = torch.empty((im_y, im_x), dtype=torch.int32, device=beads.device)
-    hw = _upload_async(disc_halfwidth_table(max(rmax, 1)), beads.device)
+    hw = upload_async(disc_halfwidth_table(max(rmax, 1)), beads.device)
     with torch.cuda.device(beads.device):
         _lib.call("mgb_bead_labels", _ptr(beads), m, int(im_y), int(im_x), _ptr(hw), max(rmax, 1), _ptr(labels),
                   _stream())

@@ -24,6 +24,7 @@ import numpy as np
 import torch
 
 from . import ops
+from .dist import allreduce_maxima
 
 
 def copy_forward_sources(num_times: int, search_timesteps) -> np.ndarray:
@@ -41,6 +42,47 @@ def copy_forward_sources(num_times: int, search_timesteps) -> np.ndarray:
         else:
             src[t] = max(s for s in search if s <= t)
     return src
+
+
+def search_centers(centers_at, num_times: int, search_timesteps):
+    """Marker centres at every search timestep, copied forward to the other timepoints
+    (find.py:143-157).  centers_at(ts) -> (x, y, fg_radius), M values each in any shape.  Returns
+    x, y (M, T) float64, the radii (M, Ts) int32 and the source timestep of every timepoint."""
+    src = copy_forward_sources(num_times, search_timesteps)
+    search = sorted(set(src.tolist()))
+    xs, ys, rs = zip(*(centers_at(ts) for ts in search))
+    column = np.searchsorted(search, src)
+    x = np.stack([np.asarray(v, dtype=np.float64).reshape(-1) for v in xs], 1)[:, column]
+    y = np.stack([np.asarray(v, dtype=np.float64).reshape(-1) for v in ys], 1)[:, column]
+    radius = np.stack([np.asarray(v).reshape(-1) for v in rs], 1).astype(np.int32)
+    return x, y, radius, src
+
+
+def upload_blocks(blocks, dst: torch.Tensor, h2d, ff: Optional[ops.FlatFieldPlan] = None, ring=None) -> int:
+    """Upload ((channel, time), block) pairs into dst[channel, time] on the copy stream `h2d`; the
+    current stream waits for each block and runs flat-field pass 1 (`ff`, skipped when absent or
+    the identity) on it as it lands.  A tensor block is copied directly (asynchronously when it is
+    pinned); an ndarray or a fill callable goes through the PinnedRing `ring`.  Returns the number
+    of blocks."""
+    compute = torch.cuda.current_stream(dst.device)
+    maxima = ff is not None and not ff.identity
+    h2d.wait_stream(compute)          # dst may be overwritten once the kernels queued before are done with it
+    if maxima:
+        ff.maxima.zero_()
+    n = 0
+    for (ci, ti), block in blocks:
+        if isinstance(block, torch.Tensor):
+            with torch.cuda.stream(h2d):
+                dst[ci, ti].copy_(block, non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record(h2d)
+        else:
+            ev = ring.send(block, dst[ci, ti], h2d)
+        compute.wait_event(ev)
+        if maxima:
+            ops.flatfield_maxima_accumulate(dst[ci, ti], ff, ci)
+        n += 1
+    return n
 
 
 @dataclass
@@ -83,73 +125,62 @@ class QuantifyPlan:
 
         x, y: (M, T) float64 centres in image coordinates for every timepoint (non-search
         timepoints hold the copied-forward centres, find.py:156-157,174-175); fg_radius
-        (M, Ts) int -- refined radius or max_button_radius per search timestep."""
-        c, t = self.tile_shape[:2]
-        dev = self.device
-        x = torch.as_tensor(np.asarray(x, dtype=np.float64)).to(dev).contiguous()
-        y = torch.as_tensor(np.asarray(y, dtype=np.float64)).to(dev).contiguous()
-        if x.dim() != 2 or x.shape[1] != t or x.shape != y.shape:
+        (M, Ts) int -- refined radius or max_button_radius per search timestep.  The boxes and
+        masks are built as `components.ButtonFinder` builds them (`components.chip_markers`)."""
+        from .components import chip_markers
+
+        t = self.tile_shape[1]
+        if np.ndim(x) != 2 or np.shape(x)[1] != t or np.shape(x) != np.shape(y):
             raise ValueError(f"x and y must have shape (M, {t})")
-        m = x.shape[0]
-        src = copy_forward_sources(t, search_timesteps)
-        search = sorted(set(src.tolist()))
-        fg_radius = np.asarray(fg_radius, dtype=np.int32).reshape(m, -1)
-        if fg_radius.shape[1] != len(search):
-            raise ValueError("fg_radius must have one column per search timestep")
-        him, wim = self.image_shape[-2:]
-        self.boxes, rel = ops.bounding_boxes(x, y, self.roi_length, wim, him, want_rel=True)
-        fgs, bgs = [], []
-        for k, ts in enumerate(search):
-            f, b = ops.chip_masks(rel[:, ts].contiguous(), torch.from_numpy(fg_radius[:, k].copy()).to(dev),
-                                  int(max_button_radius), int(chamber_radius), self.roi_length)
-            fgs.append(f)
-            bgs.append(b)
-        self.fg = torch.stack(fgs, 1).contiguous()
-        self.bg = torch.stack(bgs, 1).contiguous()
-        index = {ts: k for k, ts in enumerate(search)}
-        self.mask_t = torch.tensor([index[int(s)] for s in src], dtype=torch.int32, device=dev)
-        self.order = ops.spatial_order(self.boxes)
-        self.mask_counts = ops.mask_count_max(self.fg, self.bg) if m else (0, 0)
-        self.x, self.y = x, y
+        mk = chip_markers(x, y, fg_radius, search_timesteps, chamber_radius, max_button_radius, self.roi_length,
+                          self.image_shape, self.device)
+        self._set_markers(mk, ops.spatial_order(mk.boxes))
         return self
 
     def set_bead_markers(self, beads):
         """Beads (BeadFinder, find.py:503-605): beads (M,3) rows (row, col, radius), constant
-        over time (find.py:543-550); fg/bg from the label raster (find.py:561-586)."""
-        c, t = self.tile_shape[:2]
-        dev = self.device
-        beads = np.asarray(beads, dtype=np.float64).reshape(-1, 3)
-        m = len(beads)
-        him, wim = self.image_shape[-2:]
-        x = torch.from_numpy(np.repeat(beads[:, 1:2], t, axis=1)).to(dev).contiguous()
-        y = torch.from_numpy(np.repeat(beads[:, 0:1], t, axis=1)).to(dev).contiguous()
-        self.boxes = ops.bounding_boxes(x, y, self.roi_length, wim, him)
-        beads_i = torch.from_numpy(beads.astype(np.int64).astype(np.int32)).to(dev)   # astype(int), find.py:561
-        self.labels = ops.bead_labels(beads_i, him, wim)
-        box0 = self.boxes[:, 0].contiguous() if t > 0 else torch.zeros((m, 2), dtype=torch.int32, device=dev)
-        fg, bg = ops.bead_masks(self.labels, box0, self.roi_length)
-        self.fg, self.bg = fg[:, None].contiguous(), bg[:, None].contiguous()
-        self.mask_t = torch.zeros(t, dtype=torch.int32, device=dev)
-        self.order = ops.spatial_order(self.boxes) if t > 0 else None
-        self.mask_counts = ops.mask_count_max(self.fg, self.bg) if m else (0, 0)
-        self.x, self.y = x, y
+        over time (find.py:543-550); fg/bg from the label raster (find.py:561-586), built as
+        `components.BeadFinder` builds them (`components.bead_markers`)."""
+        from .components import bead_markers
+
+        t = self.tile_shape[1]
+        mk = bead_markers(beads, t, self.roi_length, self.image_shape, self.device)
+        self._set_markers(mk, ops.spatial_order(mk.boxes) if t > 0 else None)
+        self.labels = mk.labels
         return self
 
-    # -- device-resident run ------------------------------------------------------------------
+    def _set_markers(self, mk, order) -> None:
+        self.x, self.y, self.boxes, self.fg, self.bg, self.mask_t = mk.x, mk.y, mk.boxes, mk.fg, mk.bg, mk.mask_t
+        self.order = order
+        # exact counts, read back once: they size the gather's value lists for every run of the plan
+        self.mask_counts = ops.mask_count_max(self.fg, self.bg) if mk.boxes.shape[0] else (0, 0)
+
+    def _stage(self, record: Optional[list], name: str, fn):
+        """fn(), bracketed by CUDA events on the current stream that are appended to `record` as
+        (name, start, end) when a record list is given."""
+        if record is None:
+            return fn()
+        stream = torch.cuda.current_stream(self.device)
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record(stream)
+        out = fn()
+        b.record(stream)
+        record.append((name, a, b))
+        return out
+
     # -- markers found on the device-resident image -----------------------------------------------
-    def stitched(self, tiles: torch.Tensor, image_out=None) -> torch.Tensor:
+    def stitched(self, tiles: torch.Tensor, image_out=None, record: Optional[list] = None) -> torch.Tensor:
         """Flat-field + stitch only (the first two stages of run_device): the image the finders
         search, (C, T, Him, Wim) in HBM.  Pass it back to run_device(image=...) to skip the
-        recomputation."""
+        recomputation.  record: as in run_device."""
         ff = self.ff
         maxima = None
         if not ff.identity:
-            maxima = ops.flatfield_maxima(tiles, ff)
+            maxima = self._stage(record, "flatfield_max", lambda: ops.flatfield_maxima(tiles, ff))
             if self.group is not None:
-                import torch.distributed as dist
-
-                dist.all_reduce(maxima, op=dist.ReduceOp.MAX, group=self.group)
-        return ops.flatfield_stitch(tiles, overlap=self.overlap, plan=ff, maxima=maxima, out=image_out)
+                self._stage(record, "allreduce_max", lambda: allreduce_maxima(maxima, self.group))
+        return self._stage(record, "flatfield_stitch", lambda: ops.flatfield_stitch(
+            tiles, overlap=self.overlap, plan=ff, maxima=maxima, out=image_out))
 
     def locate_chip_markers(self, image: torch.Tensor, finder, tag, channels=None):
         """Button centres found on the device image by a `components.ButtonFinder` (GPU circle
@@ -162,17 +193,7 @@ class QuantifyPlan:
         tag = np.asarray(tag)
         names = np.asarray(channels if channels is not None else [f"c{k}" for k in range(c)])
         assay = Dataset(coords={"tag": (("mark_row", "mark_col"), tag), "channel": (("channel",), names)})
-        rows, cols = tag.shape
-        src = copy_forward_sources(t, finder.search_timesteps)
-        search = sorted(set(src.tolist()))
-        x = np.empty((rows * cols, t))
-        y = np.empty((rows * cols, t))
-        radius = np.empty((rows * cols, len(search)), dtype=np.int32)
-        for k, ts in enumerate(search):
-            xs, ys, rs = finder._gpu_centers(assay, image, ts)
-            x[:, ts], y[:, ts], radius[:, k] = xs.reshape(-1), ys.reshape(-1), rs
-        for ti in range(t):
-            x[:, ti], y[:, ti] = x[:, src[ti]], y[:, src[ti]]
+        x, y, radius, _ = search_centers(lambda ts: finder._gpu_centers(assay, image, ts), t, finder.search_timesteps)
         return self.set_chip_markers(x, y, radius, finder.chamber_radius, finder.max_button_radius,
                                      finder.search_timesteps)
 
@@ -185,6 +206,13 @@ class QuantifyPlan:
         beads = finder.find_centers(Dataset(coords={"channel": (("channel",), names)}), image)
         return self.set_bead_markers(beads)
 
+    def gather_stats(self, image: torch.Tensor, boxes: torch.Tensor, mask_t: torch.Tensor, **kwargs):
+        """`ops.roi_gather_stats` of `image` at `boxes` with the plan's masks, marker order, medians
+        and mask counts; kwargs go to it unchanged (want_roi, out_roi, out_stats, peer_stats)."""
+        return ops.roi_gather_stats(image, boxes, self.fg, self.bg, self.roi_length, mask_t=mask_t, order=self.order,
+                                    medians=self.medians, mask_counts=self.mask_counts, **kwargs)
+
+    # -- device-resident run ------------------------------------------------------------------
     def run_device(self, tiles: torch.Tensor, want_roi: bool = True, image_out=None, roi_out=None,
                    stats_out=None, record: Optional[list] = None, peer_stats=None,
                    image: Optional[torch.Tensor] = None) -> QuantifyResult:
@@ -199,35 +227,15 @@ class QuantifyPlan:
             raise RuntimeError("set_chip_markers / set_bead_markers must be called first")
         if tuple(tiles.shape) != self.tile_shape:
             raise ValueError(f"tiles have shape {tuple(tiles.shape)}, plan was built for {self.tile_shape}")
-        stream = torch.cuda.current_stream(self.device)
-
-        def stage(name, fn):
-            if record is None:
-                return fn()
-            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(stream)
-            out = fn()
-            b.record(stream)
-            record.append((name, a, b))
-            return out
-
-        ff = self.ff
         maxima = None
         if image is None:
-            if not ff.identity:
-                maxima = stage("flatfield_max", lambda: ops.flatfield_maxima(tiles, ff))
-                if self.group is not None:
-                    import torch.distributed as dist
-
-                    stage("allreduce_max", lambda: dist.all_reduce(maxima, op=dist.ReduceOp.MAX, group=self.group))
-            image = stage("flatfield_stitch", lambda: ops.flatfield_stitch(tiles, overlap=self.overlap, plan=ff,
-                                                                           maxima=maxima, out=image_out))
+            image = self.stitched(tiles, image_out, record)
+            maxima = None if self.ff.identity else self.ff.maxima
         elif tuple(image.shape) != tuple(self.image_shape):
             raise ValueError(f"image has shape {tuple(image.shape)}, plan expects {tuple(self.image_shape)}")
-        roi, stats = stage("roi_gather_stats", lambda: ops.roi_gather_stats(
-            image, self.boxes, self.fg, self.bg, self.roi_length, mask_t=self.mask_t, want_roi=want_roi,
-            out_roi=roi_out, out_stats=stats_out, order=self.order, peer_stats=peer_stats, medians=self.medians,
-            mask_counts=self.mask_counts))
+        roi, stats = self._stage(record, "roi_gather_stats", lambda: self.gather_stats(
+            image, self.boxes, self.mask_t, want_roi=want_roi, out_roi=roi_out, out_stats=stats_out,
+            peer_stats=peer_stats))
         return QuantifyResult(image, roi, self.fg, self.bg, self.mask_t, self.boxes, stats, maxima)
 
 
@@ -236,9 +244,10 @@ class HostStagedRunner:
     dask-chunk reads at find.py:121,155,590 and zarr writes at stitch.py:45, find.py:201,604).
 
     The host side owns pinned buffers: `tiles_host` (C,T,R,Cc,H,W) in, `image_host`, `roi_host`,
-    `stats_host` out.  One timepoint (all channels) is a chunk.  A copy stream moves chunk t+1
-    to the GPU while the compute stream runs flat-field pass 1 on chunk t; after the maxima
-    all-reduce, pass 2 + gather run per chunk and a second copy stream drains the results."""
+    `stats_host` out.  A copy stream moves the (channel, timepoint) blocks to the GPU while the
+    compute stream runs flat-field pass 1 on the blocks that have landed (`upload_blocks`); after
+    the maxima all-reduce, pass 2 + gather run on the whole stack and a second copy stream drains
+    the results."""
 
     def __init__(self, plan: QuantifyPlan, want_image: bool = True, want_roi: bool = True):
         self.plan = plan
@@ -272,28 +281,10 @@ class HostStagedRunner:
         this assay overlap the host->device copies of the next `run()` (PCIe is full duplex), so a
         sequence of assays is bounded by max(H2D, D2H) + compute instead of their sum.  Call
         `synchronize()` before reading the host outputs."""
-        plan = self.plan
-        c, t, r, cc, h, w = plan.tile_shape
-        compute = torch.cuda.current_stream(plan.device)
-        ff = plan.ff
-        # ---- stage in + pass 1 (per timepoint, per channel: each (c, t) block is contiguous).
-        # tiles_dev may be overwritten once the previous assay's kernels are done with it.
-        self.h2d.wait_stream(compute)
-        events = []
-        for ti in range(t):
-            with torch.cuda.stream(self.h2d):
-                for ci in range(c):
-                    self.tiles_dev[ci, ti].copy_(tiles_host[ci, ti], non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(self.h2d)
-            events.append(ev)
-        if not ff.identity:
-            ff.maxima.zero_()
-        for ti in range(t):
-            compute.wait_event(events[ti])
-            if not ff.identity:
-                for ci in range(c):
-                    ops.flatfield_maxima_accumulate(self.tiles_dev[ci, ti], ff, ci)
+        c, t = self.plan.tile_shape[:2]
+        # stage in + pass 1, time-major: each (channel, time) block is contiguous
+        upload_blocks((((ci, ti), tiles_host[ci, ti]) for ti in range(t) for ci in range(c)), self.tiles_dev,
+                      self.h2d, self.plan.ff)
         self.finish(image_host, roi_host, stats_host)
 
     def finish(self, image_host, roi_host, stats_host) -> None:
@@ -303,9 +294,7 @@ class HostStagedRunner:
         ff = plan.ff
         compute = torch.cuda.current_stream(plan.device)
         if not ff.identity and plan.group is not None:
-            import torch.distributed as dist
-
-            dist.all_reduce(ff.maxima, op=dist.ReduceOp.MAX, group=plan.group)
+            allreduce_maxima(ff.maxima, plan.group)
         # ---- pass 2 + stitch, gather + reductions on the whole resident stack.  image_dev /
         # roi_dev / stats_dev are reused: wait until the previous assay's results have left them.
         compute.wait_stream(self.d2h)
@@ -317,9 +306,8 @@ class HostStagedRunner:
             with torch.cuda.stream(self.d2h):
                 self.d2h.wait_event(done_image)
                 ops.to_host_dense(image, out=image_host)   # one pitched copy, also for a padded image
-        roi, stats = ops.roi_gather_stats(image, plan.boxes, plan.fg, plan.bg, plan.roi_length, mask_t=plan.mask_t,
-                                          want_roi=self.want_roi, out_roi=self.roi_dev, out_stats=self.stats_dev,
-                                          order=plan.order, medians=plan.medians, mask_counts=plan.mask_counts)
+        roi, stats = plan.gather_stats(image, plan.boxes, plan.mask_t, want_roi=self.want_roi, out_roi=self.roi_dev,
+                                       out_stats=self.stats_dev)
         done_roi = torch.cuda.Event()
         done_roi.record(compute)
         with torch.cuda.stream(self.d2h):
@@ -408,20 +396,8 @@ class ChunkStager:
 
     def feed(self, chunks) -> int:
         """Stage every chunk and run flat-field pass 1 on it.  Returns the number of blocks."""
-        runner, plan = self.runner, self.runner.plan
-        compute = torch.cuda.current_stream(plan.device)
-        ff = plan.ff
-        runner.h2d.wait_stream(compute)
-        if not ff.identity:
-            ff.maxima.zero_()
-        n = 0
-        for (ci, ti), block in chunks:
-            ev = self.ring.send(block, runner.tiles_dev[ci, ti], runner.h2d)
-            compute.wait_event(ev)
-            if not ff.identity:
-                ops.flatfield_maxima_accumulate(runner.tiles_dev[ci, ti], ff, ci)
-            n += 1
-        return n
+        runner = self.runner
+        return upload_blocks(chunks, runner.tiles_dev, runner.h2d, runner.plan.ff, self.ring)
 
     def close(self):
         self.ring.close()
@@ -522,9 +498,7 @@ class StreamingRunner:
                 ev.record(compute)
                 consumed[slot] = ev
             if plan.group is not None:
-                import torch.distributed as dist
-
-                dist.all_reduce(ff.maxima, op=dist.ReduceOp.MAX, group=plan.group)
+                allreduce_maxima(ff.maxima, plan.group)
         # ---- pass 2: correct + stitch + gather per timepoint, results drained behind the kernels
         drained = [None] * self.depth                # per slot: (timepoint, event after its D2H copies)
 
@@ -543,10 +517,8 @@ class StreamingRunner:
             compute.wait_event(up)
             image = ops.flatfield_stitch(self.tiles_dev[slot], overlap=plan.overlap, plan=ff,
                                          maxima=None if ff.identity else ff.maxima, out=self.image_dev[slot])
-            roi, stats = ops.roi_gather_stats(image, self.boxes_t[ti], plan.fg, plan.bg, plan.roi_length,
-                                              mask_t=self.mask_t[ti], want_roi=self.want_roi,
-                                              out_roi=self.roi_dev[slot], out_stats=self.stats_dev[slot], order=plan.order,
-                                              medians=plan.medians, mask_counts=plan.mask_counts)
+            roi, stats = plan.gather_stats(image, self.boxes_t[ti], self.mask_t[ti], want_roi=self.want_roi,
+                                           out_roi=self.roi_dev[slot], out_stats=self.stats_dev[slot])
             done = torch.cuda.Event()
             done.record(compute)
             consumed[slot] = done

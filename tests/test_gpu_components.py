@@ -193,6 +193,43 @@ def test_button_finder_multi_search_matches_reference_call(cuda_device, golden, 
     np.testing.assert_array_equal(out.y.values, g["y"])
 
 
+def test_finders_with_pinned_centres_never_synchronise(cuda_device):
+    """ButtonFinder and BeadFinder with pinned centres on the stitched image in HBM only queue
+    work: no synchronising copy or read-back, so an assay's finder never waits behind its image
+    download and the next assay's upload can be queued at once."""
+    from magnify_b200.components import BeadFinder, ButtonFinder, Stitcher
+    from magnify_b200.dataset import Assay
+    from oracle import rois as o_rois
+    from test_gpu_end_to_end import split_into_tiles
+    from test_gpu_finders import draw_chip
+
+    rows, cols, t, overlap = 3, 4, 3, 8
+    chip = draw_chip((rows, cols), 20, row_dist=100, col_dist=100) + 50                     # (400, 500)
+    tiles = np.stack([split_into_tiles(chip + 3 * k, 2, 2, overlap) for k in range(t)])[None]
+    xp = Stitcher(overlap, device=cuda_device)(Assay({"tile": (TILE_DIMS, tiles)},
+                                                     coords={"tag": (("mark_row", "mark_col"), np.full((rows, cols), "a"))}))
+    image = xp["image"].data
+    yy, xx = np.mgrid[1:rows + 1, 1:cols + 1] * 100.0
+
+    def centers(assay, ts):
+        return xx + ts, yy - ts, np.full((rows, cols), 10)
+
+    beads = np.array([[100.0, 100.0, 10.0], [200.0, 300.0, 10.0], [310.0, 420.0, 9.0]])
+    bead_assay = Assay({"image": (("channel", "time", "im_y", "im_x"), image)})
+    torch.cuda.synchronize()
+    torch.cuda.set_sync_debug_mode("error")
+    try:
+        chips = ButtonFinder(100, 100, 16, 32, 60, search_timestep=[0, 2], centers=centers, device=cuda_device)(xp)
+        found = BeadFinder(16, 24, centers=beads, device=cuda_device)(bead_assay)
+    finally:
+        torch.cuda.set_sync_debug_mode("default")
+    host = image.numpy()
+    x, y = chips.x.values, chips.y.values
+    assert (x[:, 1] == x[:, 0]).all() and (x[:, 2] == x[:, 0] + 2).all()                  # copied forward from t = 0
+    np.testing.assert_array_equal(chips.roi.values, o_rois.gather_rois(host, x, y, 72))
+    np.testing.assert_array_equal(found.roi.values, o_rois.gather_rois(host, found.x.values, found.y.values, 48))
+
+
 def test_filter_expression_and_mrbles_intensities(cuda_device):
     """SURVEY.md section 8f row N3: the consumers of the summaries (filter.py:11-37,
     identify.py:76-80) on GPU medians / means, against the NumPy restatement."""

@@ -191,7 +191,7 @@ def test_markers_located_on_device_image(cuda_device):
     """tiles in HBM -> flat-field + stitch -> buttons found on the device image -> gather + stats,
     without the image leaving the GPU; equals the component path (image through the host)."""
     from magnify_b200 import pipeline
-    from magnify_b200.components import BeadFinder, ButtonFinder
+    from magnify_b200.components import BeadFinder, ButtonFinder, summaries
     from magnify_b200.dataset import Assay
     from test_gpu_finders import draw_beads, draw_chip
     from test_gpu_end_to_end import split_into_tiles
@@ -218,7 +218,7 @@ def test_markers_located_on_device_image(cuda_device):
     fg = res.fg.cpu().numpy().astype(bool)[:, res.mask_t.cpu().numpy()]
     np.testing.assert_array_equal(fg, out.fg.values)
     assert (res.stats[:, 0, :, 4].cpu().numpy() > 900).all()                              # fg means on the buttons
-    # beads
+    # beads: the plan equals BeadFinder with the same centres on the same image
     beads_img = draw_beads((600, 500), [[100, 100], [300, 250], [500, 400]]) + 20
     tiles_b = torch.from_numpy(np.ascontiguousarray(split_into_tiles(beads_img, 2, 2, overlap)[None, None])).to(cuda_device)
     finder = BeadFinder(16, 24, num_iter=5000, device=cuda_device)
@@ -227,6 +227,16 @@ def test_markers_located_on_device_image(cuda_device):
     bplan.locate_bead_markers(bimage, finder)
     bres = bplan.run_device(tiles_b, image=bimage)
     assert bres.roi.shape[0] == 3 and (bres.stats[:, 0, 0, 4].cpu().numpy() > 900).all()
+    bassay = Assay({"image": (("channel", "time", "im_y", "im_x"), bimage.cpu().numpy())},
+                   coords={"channel": (("channel",), np.array(["c0"]))})
+    beads = finder.find_centers(bassay, bimage)
+    bout = BeadFinder(16, 24, centers=beads, device=cuda_device)(bassay)
+    np.testing.assert_array_equal(bplan.x.cpu().numpy(), bout.x.values)
+    np.testing.assert_array_equal(bres.roi.cpu().numpy(), bout.roi.values)
+    mask_t = bres.mask_t.cpu().numpy()
+    np.testing.assert_array_equal(bres.fg.cpu().numpy().astype(bool)[:, mask_t], bout.fg.values)
+    np.testing.assert_array_equal(bres.bg.cpu().numpy().astype(bool)[:, mask_t], bout.bg.values)
+    np.testing.assert_array_equal(bres.stats.cpu().numpy(), summaries(bout, device=cuda_device).cpu().numpy())
 
 
 @pytest.mark.parametrize("identity", [False, True])
