@@ -31,6 +31,14 @@ __host__ __device__ inline bool aligned16(const void* p) {
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// ceil(2^32 / d): the copy loops divide an index x by d as __umulhi(x, magic_u32(d)).  d = 1 has no
+// 32-bit value, so a loop that divides by d is never chosen for d = 1.
+inline uint32_t magic_u32(uint32_t d) { return (uint32_t)((0x100000000ULL + d - 1) / d); }
+
+// Doubles per summary record of (marker, channel, time):
+// n_fg, n_bg, sum_fg, sum_bg, mean_fg, mean_bg, median_fg, median_bg.
+constexpr int kStatsRec = 8;
+
 // Stream-ordered scratch for the few entry points whose temporary sizes are only known inside the
 // call (CUB temp storage, the unique-circle list, large-mask workspaces).  The blocks come from a
 // PRIVATE memory pool per device, created on first use, that keeps at most 1 GiB of freed blocks

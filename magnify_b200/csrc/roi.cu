@@ -6,7 +6,7 @@
 // One CTA copies one ROI (m,c,t); CTAs are numbered in roi memory order so consecutive CTAs
 // write consecutive 2*L*L-byte blocks.  Reductions ride on the copy: the pixels are already in
 // registers, the masks (shared by all channels / copy-forward timepoints) come from L2.
-#include "common.cuh"
+#include "roi_stage.cuh"
 
 namespace mgb {
 
@@ -57,8 +57,6 @@ struct GatherParams {
   const uint8_t* bg;
   double* stats;
 };
-
-constexpr int kRec = 8;   // doubles per summary record: n_fg n_bg sum_fg sum_bg mean_fg mean_bg median_fg median_bg
 
 __device__ __forceinline__ uint64_t block_sum_u64(uint64_t v, uint64_t* smem) {
 #pragma unroll
@@ -134,7 +132,7 @@ __global__ void __launch_bounds__(kThreads) roi_gather_words_kernel(const Gather
     const uint64_t b = block_sum_u64(s_bg, red[1]);
     const uint64_t na = block_sum_u64(n_fg, red[2]);
     const uint64_t nb = block_sum_u64(n_bg, red[3]);
-    if (threadIdx.x == 0) write_record(p.stats + n * kRec, na, nb, a, b);
+    if (threadIdx.x == 0) write_record(p.stats + n * kStatsRec, na, nb, a, b);
   }
 }
 
@@ -182,7 +180,7 @@ roi_gather_scalar_kernel(const U* __restrict__ image, U* __restrict__ roi, int64
     const uint64_t b = block_sum_u64(s_bg, red[1]);
     const uint64_t na = block_sum_u64(n_fg, red[2]);
     const uint64_t nb = block_sum_u64(n_bg, red[3]);
-    if (threadIdx.x == 0) write_record(stats + n * kRec, na, nb, a, b);
+    if (threadIdx.x == 0) write_record(stats + n * kStatsRec, na, nb, a, b);
   }
 }
 
@@ -381,30 +379,13 @@ roi_stats_f32_kernel(const float* __restrict__ roi, int64_t C, int64_t T, int L,
     double s[4] = {0.0, 0.0, 0.0, 0.0};
     for (int w = 0; w < kThreads / 32; ++w)
       for (int k = 0; k < 4; ++k) s[k] += red[k][w];
-    double* out = stats + n * kRec;
+    double* out = stats + n * kStatsRec;
     out[0] = s[0]; out[1] = s[1]; out[2] = s[2]; out[3] = s[3];
     out[4] = s[2] / s[0];   // 0 / 0 = NaN for an empty mask, like np.nanmean
     out[5] = s[3] / s[1];
     out[6] = out[7] = __longlong_as_double(0x7ff8000000000000LL);   // medians: filled by the median kernel
   }
 }
-
-static uint32_t magic_for(uint32_t d) { return (uint32_t)((0x100000000ULL + d - 1) / d); }
-
-// roi_tma.cu
-int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64_t H, int64_t W, int itemsize,
-                   const int32_t* boxes, const int32_t* order, const int32_t* mask_t, int64_t Tm, const uint8_t* fg,
-                   const uint8_t* bg, int64_t M, int L, void* roi, double* stats, const uint64_t* host_peers,
-                   int n_peers, cudaStream_t st);
-
-// roi_lists.cu
-int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int64_t H, int64_t W,
-                     const int32_t* boxes, const int32_t* order, const int32_t* mask_t, int64_t Tm, const uint8_t* fg,
-                     const uint8_t* bg, int64_t M, int L, void* roi, double* stats, int want_median, int nf_max,
-                     int nb_max, const uint64_t* host_peers, int n_peers, cudaStream_t st);
-
-extern int g_gather_loader;
-extern int g_gather_wpm;
 
 static int g_tma_enabled = 1;
 
@@ -448,63 +429,59 @@ int mgb_bounding_boxes(const double* x, const double* y, int64_t n, int L, int64
   return MGB_OK;
 }
 
-static int gather_common(const void* image, int64_t image_pitch, int64_t C, int64_t T, int64_t H, int64_t W,
-                         int itemsize, const int32_t* boxes, const int32_t* order, int64_t marker_stride, const int32_t* mask_t, int64_t Tm, const uint8_t* fg,
-                         const uint8_t* bg, int64_t M, int L, void* roi, double* stats,
-                         cudaStream_t st, const uint64_t* host_peers = nullptr, int n_peers = 0,
-                         int want_median = 0, int nf_max = -1, int nb_max = -1, int* host_median_done = nullptr) {
-  if (host_median_done) *host_median_done = 0;
-  const bool with_stats = stats != nullptr;
+static int gather_common(const GatherArgs& a, cudaStream_t st, int* host_median_done = nullptr) {
+  const int64_t C = a.C, T = a.T, H = a.H, W = a.W, M = a.M;
+  const int L = a.L, itemsize = a.itemsize;
   if (M < 0 || C < 0 || T < 0 || L <= 0 || H < L || W < L) return MGB_EINVAL;
-  const int64_t pitch = image_pitch > 0 ? image_pitch : W;   // row pitch in elements
+  const int64_t pitch = a.row_pitch();   // row pitch in elements
   if (pitch < W) return MGB_EINVAL;
   if (itemsize != 1 && itemsize != 2 && itemsize != 4 && itemsize != 8) return MGB_EINVAL;
   if (L > 4096) return MGB_EUNSUPPORTED;
   const int64_t n_roi = M * C * T;
   if (n_roi == 0) return MGB_OK;
   if (n_roi > INT32_MAX) return MGB_EUNSUPPORTED;
-  if (!image || (!boxes && marker_stride == 0) || (!roi && !with_stats)) return MGB_EINVAL;
-  if (with_stats && (!mask_t || !fg || !bg || Tm <= 0 || itemsize != 2)) return MGB_EINVAL;
-  if (g_tma_enabled && marker_stride == 0 && with_stats && nf_max >= 0 && nb_max >= 0) {
+  if (!a.image || (!a.boxes && a.marker_stride == 0) || (!a.roi && !a.with_stats)) return MGB_EINVAL;
+  if (a.with_stats && (!a.mask_t || !a.fg || !a.bg || a.Tm <= 0 || itemsize != 2)) return MGB_EINVAL;
+  if (g_tma_enabled && a.marker_stride == 0 && a.with_stats && a.nf_max >= 0 && a.nb_max >= 0) {
     // masked-value lists: sums, means and (optionally) medians in the gather (roi_lists.cu)
-    const int rc = roi_gather_lists(image, pitch, C, T, H, W, boxes, order, mask_t, Tm, fg, bg, M, L, roi, stats,
-                                    want_median, nf_max, nb_max, host_peers, n_peers, st);
-    if (rc == MGB_OK && want_median && host_median_done) *host_median_done = 1;
+    const int rc = roi_gather_lists(a, st);
+    if (rc == MGB_OK && a.want_median && host_median_done) *host_median_done = 1;
     if (rc != MGB_EALIGN) return rc;
   }
-  if (g_tma_enabled && marker_stride == 0) {
+  if (g_tma_enabled && a.marker_stride == 0) {
     // TMA-staged path (roi_tma.cu); MGB_EALIGN means "not applicable here", fall through.
-    const int rc = roi_gather_tma(image, pitch, C, T, H, W, itemsize, boxes, order, mask_t, Tm, fg, bg, M, L, roi, stats,
-                                  host_peers, n_peers, st);
+    const int rc = roi_gather_tma(a, st);
     if (rc != MGB_EALIGN) return rc;
   }
-  if (n_peers > 0) return MGB_EUNSUPPORTED;   // peer write-out exists only in the staged kernels
+  if (a.n_peers > 0) return MGB_EUNSUPPORTED;   // peer write-out exists only in the staged kernels
   const int unit = itemsize / 2;
   const int Lu = L * (unit ? unit : 1);
-  // (Lu > 2: a row of one word has no 32-bit multiply-high magic number for its division)
-  const bool word_path = itemsize >= 2 && (Lu % 2 == 0) && Lu > 2 &&
-                         ((reinterpret_cast<uintptr_t>(image) & 3u) == 0) &&
-                         (!roi || (reinterpret_cast<uintptr_t>(roi) & 3u) == 0) &&
-                         (!with_stats || ((reinterpret_cast<uintptr_t>(fg) & 1u) == 0 &&
-                                          (reinterpret_cast<uintptr_t>(bg) & 1u) == 0));
+  const bool word_path = itemsize >= 2 && word_rows(Lu) &&
+                         ((reinterpret_cast<uintptr_t>(a.image) & 3u) == 0) &&
+                         (!a.roi || (reinterpret_cast<uintptr_t>(a.roi) & 3u) == 0) &&
+                         (!a.with_stats || ((reinterpret_cast<uintptr_t>(a.fg) & 1u) == 0 &&
+                                            (reinterpret_cast<uintptr_t>(a.bg) & 1u) == 0));
   if (word_path) {
     GatherParams p{};
-    p.image = (const uint16_t*)image; p.roi = (uint16_t*)roi;
-    p.C = C; p.T = T; p.H = H; p.W = pitch * unit; p.boxes = boxes; p.marker_stride = marker_stride * unit;
+    p.image = (const uint16_t*)a.image; p.roi = (uint16_t*)a.roi;
+    p.C = C; p.T = T; p.H = H; p.W = pitch * unit; p.boxes = a.boxes; p.marker_stride = a.marker_stride * unit;
     p.unit = unit; p.L = L; p.Lu = Lu;
-    p.half = (uint32_t)(Lu / 2); p.magic = magic_for(p.half); p.words = (uint32_t)L * p.half;
-    p.mask_t = mask_t; p.Tm = Tm; p.fg = fg; p.bg = bg; p.stats = stats;
-    if (with_stats) roi_gather_words_kernel<true><<<(unsigned)n_roi, kThreads, 0, st>>>(p);
+    p.half = (uint32_t)(Lu / 2); p.magic = magic_u32(p.half); p.words = (uint32_t)L * p.half;
+    p.mask_t = a.mask_t; p.Tm = a.Tm; p.fg = a.fg; p.bg = a.bg; p.stats = a.stats;
+    if (a.with_stats) roi_gather_words_kernel<true><<<(unsigned)n_roi, kThreads, 0, st>>>(p);
     else roi_gather_words_kernel<false><<<(unsigned)n_roi, kThreads, 0, st>>>(p);
-  } else if (with_stats) {
+  } else if (a.with_stats) {
     roi_gather_scalar_kernel<uint16_t, true><<<(unsigned)n_roi, kThreads, 0, st>>>(
-        (const uint16_t*)image, (uint16_t*)roi, C, T, H, pitch, boxes, marker_stride, L, mask_t, Tm, fg, bg, stats);
+        (const uint16_t*)a.image, (uint16_t*)a.roi, C, T, H, pitch, a.boxes, a.marker_stride, L, a.mask_t, a.Tm, a.fg,
+        a.bg, a.stats);
   } else {
+    const int32_t* boxes = a.boxes;
+    const int64_t ms = a.marker_stride;
     switch (itemsize) {
-      case 1: roi_gather_scalar_kernel<uint8_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint8_t*)image, (uint8_t*)roi, C, T, H, pitch, boxes, marker_stride, L, nullptr, 0, nullptr, nullptr, nullptr); break;
-      case 2: roi_gather_scalar_kernel<uint16_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint16_t*)image, (uint16_t*)roi, C, T, H, pitch, boxes, marker_stride, L, nullptr, 0, nullptr, nullptr, nullptr); break;
-      case 4: roi_gather_scalar_kernel<uint32_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint32_t*)image, (uint32_t*)roi, C, T, H, pitch, boxes, marker_stride, L, nullptr, 0, nullptr, nullptr, nullptr); break;
-      default: roi_gather_scalar_kernel<uint64_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint64_t*)image, (uint64_t*)roi, C, T, H, pitch, boxes, marker_stride, L, nullptr, 0, nullptr, nullptr, nullptr); break;
+      case 1: roi_gather_scalar_kernel<uint8_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint8_t*)a.image, (uint8_t*)a.roi, C, T, H, pitch, boxes, ms, L, nullptr, 0, nullptr, nullptr, nullptr); break;
+      case 2: roi_gather_scalar_kernel<uint16_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint16_t*)a.image, (uint16_t*)a.roi, C, T, H, pitch, boxes, ms, L, nullptr, 0, nullptr, nullptr, nullptr); break;
+      case 4: roi_gather_scalar_kernel<uint32_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint32_t*)a.image, (uint32_t*)a.roi, C, T, H, pitch, boxes, ms, L, nullptr, 0, nullptr, nullptr, nullptr); break;
+      default: roi_gather_scalar_kernel<uint64_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint64_t*)a.image, (uint64_t*)a.roi, C, T, H, pitch, boxes, ms, L, nullptr, 0, nullptr, nullptr, nullptr); break;
     }
   }
   MGB_CUDA_LAUNCH_CHECK();
@@ -531,8 +508,10 @@ int mgb_roi_gather(const void* image, int64_t image_pitch, int64_t C, int64_t T,
                    int itemsize, const int32_t* boxes, const int32_t* order, int64_t M, int L, void* roi,
                    void* stream) {
   if (!roi && M * C * T > 0) return MGB_EINVAL;
-  return gather_common(image, image_pitch, C, T, H, W, itemsize, boxes, order, 0, nullptr, 0, nullptr, nullptr, M, L, roi,
-                       nullptr, (cudaStream_t)stream);
+  GatherArgs a{};
+  a.image = image; a.pitch = image_pitch; a.C = C; a.T = T; a.H = H; a.W = W; a.itemsize = itemsize;
+  a.boxes = boxes; a.order = order; a.M = M; a.L = L; a.roi = roi;
+  return gather_common(a, (cudaStream_t)stream);
 }
 
 int mgb_roi_gather_stats_u16(const uint16_t* image, int64_t image_pitch, int64_t C, int64_t T, int64_t H,
@@ -542,8 +521,12 @@ int mgb_roi_gather_stats_u16(const uint16_t* image, int64_t image_pitch, int64_t
                              int* host_median_done, void* stream) {
   if (host_median_done) *host_median_done = 0;
   if (!stats && M * C * T > 0) return MGB_EINVAL;
-  return gather_common(image, image_pitch, C, T, H, W, 2, boxes, order, 0, mask_t, Tm, fg, bg, M, L, roi, stats,
-                       (cudaStream_t)stream, nullptr, 0, want_median, fg_count_max, bg_count_max, host_median_done);
+  GatherArgs a{};
+  a.image = image; a.pitch = image_pitch; a.C = C; a.T = T; a.H = H; a.W = W; a.itemsize = 2;
+  a.boxes = boxes; a.order = order; a.M = M; a.L = L; a.roi = roi;
+  a.mask_t = mask_t; a.Tm = Tm; a.fg = fg; a.bg = bg; a.with_stats = true; a.stats = stats;
+  a.want_median = want_median; a.nf_max = fg_count_max; a.nb_max = bg_count_max;
+  return gather_common(a, (cudaStream_t)stream, host_median_done);
 }
 
 int mgb_roi_gather_stats_peers_u16(const uint16_t* image, int64_t image_pitch, int64_t C, int64_t T, int64_t H,
@@ -554,18 +537,23 @@ int mgb_roi_gather_stats_peers_u16(const uint16_t* image, int64_t image_pitch, i
   if (host_median_done) *host_median_done = 0;
   if (!host_peer_stats || n_peers < 1 || n_peers > 8) return MGB_EINVAL;
   if (M * C * T == 0) return MGB_OK;
-  // `stats` only flags "with summaries" here; every record is written through the peer pointers
-  return gather_common(image, image_pitch, C, T, H, W, 2, boxes, order, 0, mask_t, Tm, fg, bg, M, L, roi,
-                       reinterpret_cast<double*>(host_peer_stats[0]), (cudaStream_t)stream, host_peer_stats, n_peers,
-                       want_median, fg_count_max, bg_count_max, host_median_done);
+  GatherArgs a{};
+  a.image = image; a.pitch = image_pitch; a.C = C; a.T = T; a.H = H; a.W = W; a.itemsize = 2;
+  a.boxes = boxes; a.order = order; a.M = M; a.L = L; a.roi = roi;
+  a.mask_t = mask_t; a.Tm = Tm; a.fg = fg; a.bg = bg; a.with_stats = true; a.peers = host_peer_stats; a.n_peers = n_peers;
+  a.want_median = want_median; a.nf_max = fg_count_max; a.nb_max = bg_count_max;
+  return gather_common(a, (cudaStream_t)stream, host_median_done);
 }
 
 int mgb_roi_stats_u16(const uint16_t* roi, int64_t M, int64_t C, int64_t T, int L, const int32_t* mask_t,
                       int64_t Tm, const uint8_t* fg, const uint8_t* bg, double* stats, void* stream) {
   if (!stats && M * C * T > 0) return MGB_EINVAL;
   // every marker's roi block (C,T,L,L) is read as its own little image with the box at the origin
-  return gather_common(roi, 0, C, T, L, L, 2, nullptr, nullptr, C * T * (int64_t)L * L, mask_t, Tm, fg, bg, M, L, nullptr,
-                       stats, (cudaStream_t)stream);
+  GatherArgs a{};
+  a.image = roi; a.C = C; a.T = T; a.H = L; a.W = L; a.itemsize = 2; a.marker_stride = C * T * (int64_t)L * L;
+  a.M = M; a.L = L;
+  a.mask_t = mask_t; a.Tm = Tm; a.fg = fg; a.bg = bg; a.with_stats = true; a.stats = stats;
+  return gather_common(a, (cudaStream_t)stream);
 }
 
 int mgb_roi_median_u16(const uint16_t* roi, int64_t M, int64_t C, int64_t T, int L,

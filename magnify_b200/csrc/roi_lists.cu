@@ -249,20 +249,10 @@ roi_gather_lists_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGathe
   __shared__ uint32_t s_cnt[2];
 
   if (warp == 0) {
-    int n = 0;
-    for (int64_t base = 0; base < p.T; base += 32) {
-      const int64_t t = base + lane;
-      const bool hit = (t < p.T) && p.mask_t[t] == tm;
-      const unsigned bal = __ballot_sync(0xffffffffu, hit);
-      if (hit) tlist[n + __popc(bal & ((1u << lane) - 1))] = (int32_t)t;
-      n += __popc(bal);
-    }
+    const int n = list_timepoints<true>(p, tm, tlist, lane);
     if (lane == 0) { s_nt = n; s_cnt[0] = 0; s_cnt[1] = 0; }
   }
-  if (lane == 0) {
-    for (int s = 0; s < p.n_stages; ++s) mbar_init(smem_u32(&bars[warp * 4 + s]), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
+  if (lane == 0) init_stage_barriers(&bars[warp * 4], p.n_stages);
   __syncthreads();
 
   // CTA layout: CTA b < split_from works on all the windows of marker b; the markers from
@@ -338,14 +328,8 @@ roi_gather_lists_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGathe
     while (cur.k >= nt) { cur.k -= nt; ++cur.c; }
   };
   auto issue_tma = [&](const Cursor& cur, int s) {
-    if (lane == 0) {
-      const int64_t t = tlist[cur.k];
-      const int32_t top = p.boxes[(m * p.T + t) * 2];
-      const int32_t left = p.boxes[(m * p.T + t) * 2 + 1];
-      const uint32_t bar = my_bar0 + s * 8;
-      mbar_expect_tx(bar, tx_bytes);
-      tma_load_3d(my_stage0 + s * p.stage_bytes, &tmap, bar, left & ~7, top, (int)(cur.c * p.T + t));
-    }
+    if (lane == 0)   // uint16 images only: one 16-bit unit per pixel
+      load_window(&tmap, p, 1, m, cur.c, tlist[cur.k], my_stage0 + s * p.stage_bytes, my_bar0 + s * 8, tx_bytes);
   };
 
   Cursor ahead{0, 0, 0}, cur{0, 0, 0};
@@ -502,77 +486,42 @@ mask_count_max_kernel(const uint8_t* __restrict__ fg, const uint8_t* __restrict_
   }
 }
 
-PFN_cuTensorMapEncodeTiled get_encode_fn();   // roi_tma.cu
-extern int g_gather_wpm;
-
-static uint32_t magic_u32_(uint32_t d) { return (uint32_t)((0x100000000ULL + d - 1) / d); }
-
 // Returns MGB_OK when launched, MGB_EALIGN when this path does not apply (the caller falls back
 // to the dp2a kernels, which leave the median columns NaN), or an error.
-int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int64_t H, int64_t W,
-                     const int32_t* boxes, const int32_t* order, const int32_t* mask_t, int64_t Tm, const uint8_t* fg,
-                     const uint8_t* bg, int64_t M, int L, void* roi, double* stats, int want_median, int nf_max,
-                     int nb_max, const uint64_t* host_peers, int n_peers, cudaStream_t st) {
-  if (!stats || nf_max < 0 || nb_max < 0) return MGB_EALIGN;
-  if (nf_max > kNFL * 32 || nb_max > kNBL * 32) return MGB_EALIGN;
-  const int wu = L;
-  const int wpu = (wu + 7 + 7) & ~7;
-  if ((pitch * 2) % 16 != 0 || !aligned16(image) || wpu > 256 || L > 256) return MGB_EALIGN;
-  if ((int64_t)(L - 1) * wpu + L + 8 > 65535) return MGB_EALIGN;      // list entries are 16-bit offsets
-  if (C * T > INT32_MAX || H > INT32_MAX || pitch > INT32_MAX || M > INT32_MAX || Tm > 65535) return MGB_EALIGN;
-  PFN_cuTensorMapEncodeTiled encode = get_encode_fn();
-  if (!encode) return MGB_EALIGN;
-
-  TmaGatherParams p{};
-  p.roi = (uint16_t*)roi; p.boxes = boxes; p.order = order; p.mask_t = mask_t; p.fg = fg; p.bg = bg; p.stats = stats;
-  p.C = C; p.T = T; p.Tm = Tm; p.rows = L; p.wu = wu; p.wpu = wpu; p.unit = 1;
-  p.n_peers = 0;
-  if (host_peers && n_peers > 0) {
-    if (n_peers > 8) return MGB_EINVAL;
-    p.n_peers = n_peers;
-    for (int j = 0; j < n_peers; ++j) p.peer_stats[j] = reinterpret_cast<double*>(host_peers[j]);
-  }
-  p.stage_bytes = (L * wpu * 2 + 127) & ~127;
-  p.cap_f = (std::max(nf_max, 1) + 255) & ~255;     // whole groups of 8 slots per lane
-  p.cap_b = (std::max(nb_max, 1) + 255) & ~255;
-  p.want_median = want_median ? 1 : 0;
-  p.store = roi ? 1 : 0;
-  const bool out16 = !roi || aligned16(roi);
-  const bool out8 = !roi || (reinterpret_cast<uintptr_t>(roi) & 7u) == 0;
-  const bool out4 = !roi || (reinterpret_cast<uintptr_t>(roi) & 3u) == 0;
+int roi_gather_lists(const GatherArgs& a, cudaStream_t st) {
+  if (a.nf_max > kNFL * 32 || a.nb_max > kNBL * 32) return MGB_EALIGN;
+  StagedWindow w;
+  const int rc = stage_window(a, w);
+  if (rc != MGB_OK) return rc;
+  TmaGatherParams& p = w.p;
+  const int64_t C = a.C, T = a.T, Tm = a.Tm, M = a.M;
+  const int L = a.L, wu = p.wu;
+  if ((int64_t)(L - 1) * p.wpu + L + 8 > 65535) return MGB_EALIGN;      // list entries are 16-bit offsets
+  p.cap_f = (std::max(a.nf_max, 1) + 255) & ~255;     // whole groups of 8 slots per lane
+  p.cap_b = (std::max(a.nb_max, 1) + 255) & ~255;
+  p.want_median = a.want_median ? 1 : 0;
+  p.store = a.roi ? 1 : 0;
   int vpl = 0, qpl = 0;
-  // the copy loops divide by vpr / half with a multiply-high by ceil(2^32 / d), which has no 32-bit
-  // value for d = 1: rows of one vector (L = 8) take the quads, rows of one word (L = 2) the generic loop
-  if (wu % 8 == 0 && wu > 8 && out16) {
-    p.vpr = (uint32_t)(wu / 8);
-    p.magic_vpr = magic_u32_(p.vpr);
+  const CopyLoop loop = choose_copy_loop(p, a.roi, true);
+  if (loop == CopyLoop::kVector) {
     const int v = (int)((L * p.vpr + 31) / 32);
     vpl = v <= 12 ? 12 : v <= 21 ? 21 : v <= 36 ? 36 : 0;
-  } else if (wu % 2 == 0 && (L * wu) % 4 == 0 && out8 && (L * wu / 4 + 31) / 32 <= 24) {
+  } else if (loop == CopyLoop::kQuad) {
     qpl = (L * wu / 4 + 31) / 32 <= 12 ? 12 : 24;
-  } else if (wu % 2 == 0 && wu > 2 && out4) {
-    p.half = (uint32_t)(wu / 2);
-    p.magic_half = magic_u32_(p.half);
   }
 
   // Work layout: one CTA per marker when every marker has many windows, one warp per marker
   // when it has few and there are enough markers to fill the machine.
   const int64_t items = C * std::max<int64_t>(1, T / std::max<int64_t>(1, Tm));
-  int dev = 0, max_smem = 0, sms = 0;
-  MGB_CUDA_TRY(cudaGetDevice(&dev));
-  MGB_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-  MGB_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   // (a warp per marker needs many more markers than warp slots, else the last wave runs half empty:
   // 1792 markers on 148 x 12 slots took 2.25 ms in that layout against 1.15 ms with a CTA per marker.
   // Handing every warp an equal run of the flattened (marker, window) space instead was tried and
   // is slower still -- 3.9 ms against 2.0 ms at config 3, 14.1 against 10.3 ms at config 5 T = 4:
   // 1776 warps then write crops into 1776 regions megabytes apart at once.)
-  bool wpm = g_gather_wpm && items < 128 && M * Tm >= (int64_t)sms * 12 * 8;
+  bool wpm = g_gather_wpm && items < 128 && M * Tm >= (int64_t)w.sms * 12 * 8;
   if (const char* e = getenv("MGB_GATHER_LAYOUT")) wpm = atoi(e) == 1 ? true : atoi(e) == 0 ? false : wpm;   // tuning only
 
   const size_t list_bytes = (size_t)(p.cap_f + p.cap_b) * sizeof(uint16_t);
-  int sm_smem = 0;
-  MGB_CUDA_TRY(cudaDeviceGetAttribute(&sm_smem, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev));
   int nw = 0, ns = 0;
   size_t smem_bytes = 0;
   // warps per CTA x stages per warp: more warps hide the latency of the per-window reductions,
@@ -593,7 +542,7 @@ int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int
       const size_t fixed = (wpm ? cand : 1) * list_bytes + (size_t)cand * kHistWords * sizeof(uint32_t) +
                            (size_t)cand * 4 * sizeof(uint64_t) + (size_t)T * sizeof(int32_t) + 128;
       // 6 warps: two CTAs share an SM (half of its shared memory each, 1 KB reserved per CTA)
-      const size_t room = cand == 6 ? (size_t)(sm_smem / 2 - 1024) : (size_t)max_smem;
+      const size_t room = cand == 6 ? (size_t)(w.sm_smem / 2 - 1024) : (size_t)w.max_smem;
       if (room < fixed + 1024) continue;
       const bool one = cand >= 12 || cand == 6;
       const int n = (int)std::min<size_t>(one ? 1 : 4, (room - fixed - 1024) / ((size_t)cand * p.stage_bytes));
@@ -605,22 +554,9 @@ int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int
   bool split_tail = true;
   if (const char* e = getenv("MGB_GATHER_SPLIT")) split_tail = atoi(e) != 0;   // tuning / tests only
   p.n_stages = ns;
-  p.magic_wu = magic_u32_((uint32_t)wu);
+  p.magic_wu = magic_u32((uint32_t)wu);
 
-  CUtensorMap tmap;
-  const cuuint64_t gdim[3] = {(cuuint64_t)pitch, (cuuint64_t)H, (cuuint64_t)(C * T)};
-  const cuuint64_t gstride[2] = {(cuuint64_t)pitch * 2, (cuuint64_t)H * pitch * 2};
-  const cuuint32_t box[3] = {(cuuint32_t)wpu, (cuuint32_t)L, 1};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  const CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 3, const_cast<void*>(image), gdim, gstride, box,
-                             estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                             CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) return MGB_EALIGN;
-  p.image = (const uint16_t*)image;
-  p.H = H;
-  p.Wu = pitch;
-
-  const uint32_t magic_l = magic_u32_((uint32_t)L);
+  const uint32_t magic_l = magic_u32((uint32_t)L);
   // CTA layout: with M markers on `slots` resident CTAs the last M % slots markers would run as a
   // wave that leaves most SMs idle for a whole marker's duration (config 3: 1792 = 12 x 148 + 16).
   // Those markers are split over up to 8 CTAs each, so that the last wave is short.
@@ -634,7 +570,7 @@ int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int
     if (!WP && split_tail) {                                                                          \
       int resident = 1;                                                                                   \
       MGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident, kern, nw * 32, smem_bytes));  \
-      const int64_t slots = (int64_t)std::max(resident, 1) * sms, tail = (M * Tm) % slots;                \
+      const int64_t slots = (int64_t)std::max(resident, 1) * w.sms, tail = (M * Tm) % slots;              \
       const int64_t rounds = (items + nw - 1) / nw;                                                       \
       const int parts = (int)std::min<int64_t>({8, tail ? slots / tail : 1, rounds});                     \
       if (Tm == 1 && M > slots && parts >= 2) {                                                           \
@@ -643,7 +579,7 @@ int roi_gather_lists(const void* image, int64_t pitch, int64_t C, int64_t T, int
         grid.x = (unsigned)(p.split_from + tail * parts);                                                 \
       }                                                                                                   \
     }                                                                                                     \
-    kern<<<grid, nw * 32, smem_bytes, st>>>(tmap, p, M, magic_l);                                         \
+    kern<<<grid, nw * 32, smem_bytes, st>>>(w.tmap, p, M, magic_l);                                       \
   } while (0)
 #define MGB_LAUNCH_NW(VP, QP, WP)                       \
   do {                                                  \

@@ -42,16 +42,8 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
   __shared__ int s_nt;
   __shared__ uint32_t s_cnt[2][kTmaMaxWarps];
 
-  // timepoints whose mask timestep is tm (all of them when there are no masks)
   if (warp == 0) {
-    int n = 0;
-    for (int64_t base = 0; base < p.T; base += 32) {
-      const int64_t t = base + lane;
-      const bool hit = (t < p.T) && (!STATS || p.mask_t[t] == tm);
-      const unsigned bal = __ballot_sync(0xffffffffu, hit);
-      if (hit) tlist[n + __popc(bal & ((1u << lane) - 1))] = (int32_t)t;
-      n += __popc(bal);
-    }
+    const int n = list_timepoints<STATS>(p, tm, tlist, lane);
     if (lane == 0) s_nt = n;
   }
   if constexpr (STATS) {
@@ -76,10 +68,7 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
     nb = __reduce_add_sync(0xffffffffu, nb);
     if (lane == 0) { s_cnt[0][warp] = nf; s_cnt[1][warp] = nb; }
   }
-  if (p.loader == 0 && lane == 0) {
-    for (int s = 0; s < p.n_stages; ++s) mbar_init(smem_u32(&bars[warp * 8 + s]), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
+  if (p.loader == 0 && lane == 0) init_stage_barriers(&bars[warp * 8], p.n_stages);
   __syncthreads();
   const int nt = s_nt;
   const int n_items = nt * (int)p.C;           // item i -> (c = i / nt, t = tlist[i % nt])
@@ -129,11 +118,7 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
     if (lane == 0) {
       int64_t c, t;
       item_ct(i, &c, &t);
-      const int32_t top = p.boxes[(m * p.T + t) * 2];
-      const int32_t left = p.boxes[(m * p.T + t) * 2 + 1];
-      const uint32_t bar = my_bar0 + s * 8;
-      mbar_expect_tx(bar, tx_bytes);
-      tma_load_3d(my_stage0 + s * p.stage_bytes, &tmap, bar, (left * p.unit) & ~7, top, (int)(c * p.T + t));
+      load_window(&tmap, p, p.unit, m, c, t, my_stage0 + s * p.stage_bytes, my_bar0 + s * 8, tx_bytes);
     }
   };
   // LSU loader: the warp streams the window's 16-byte chunks with cp.async (32-byte sector
@@ -252,20 +237,10 @@ roi_gather_wpm_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
   int32_t* tlist = reinterpret_cast<int32_t*>(bars + kTmaMaxWarps * 8);
   __shared__ int s_nt;
   if (warp == 0) {
-    int n = 0;
-    for (int64_t base = 0; base < p.T; base += 32) {
-      const int64_t t = base + lane;
-      const bool hit = (t < p.T) && (!STATS || p.mask_t[t] == tm);
-      const unsigned bal = __ballot_sync(0xffffffffu, hit);
-      if (hit) tlist[n + __popc(bal & ((1u << lane) - 1))] = (int32_t)t;
-      n += __popc(bal);
-    }
+    const int n = list_timepoints<STATS>(p, tm, tlist, lane);
     if (lane == 0) s_nt = n;
   }
-  if (lane == 0) {
-    for (int s = 0; s < p.n_stages; ++s) mbar_init(smem_u32(&bars[warp * 8 + s]), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
+  if (lane == 0) init_stage_barriers(&bars[warp * 8], p.n_stages);
   __syncthreads();
   const int64_t mi = (int64_t)blockIdx.x * nw + warp;
   if (mi >= M) return;
@@ -317,11 +292,7 @@ roi_gather_wpm_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
     if (lane == 0) {
       int64_t c, t;
       item_ct(i, &c, &t);
-      const int32_t top = p.boxes[(m * p.T + t) * 2];
-      const int32_t left = p.boxes[(m * p.T + t) * 2 + 1];
-      const uint32_t bar = my_bar0 + s * 8;
-      mbar_expect_tx(bar, tx_bytes);
-      tma_load_3d(my_stage0 + s * p.stage_bytes, &tmap, bar, (left * p.unit) & ~7, top, (int)(c * p.T + t));
+      load_window(&tmap, p, p.unit, m, c, t, my_stage0 + s * p.stage_bytes, my_bar0 + s * 8, tx_bytes);
     }
   };
   for (int s = 0; s < p.n_stages - 1; ++s)
@@ -373,69 +344,23 @@ roi_gather_wpm_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
   }
 }
 
-PFN_cuTensorMapEncodeTiled get_encode_fn() {
-  static PFN_cuTensorMapEncodeTiled fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(ptr);
-  }
-  return fn;
-}
-
 int g_gather_wpm = 1;      // warp-per-marker kernel for many-marker shapes (tuning switch)
 int g_gather_loader = 0;   // 0 = TMA tensor copies (default), 1 = cp.async chunks; equal within 1% on B200
 
-static uint32_t magic_u32(uint32_t d) { return (uint32_t)((0x100000000ULL + d - 1) / d); }
-
 // Returns MGB_OK when launched, MGB_EALIGN when this path does not apply (caller falls back to
 // the LSU kernels of roi.cu), or an error.
-int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64_t H, int64_t W, int itemsize,
-                   const int32_t* boxes, const int32_t* order, const int32_t* mask_t, int64_t Tm, const uint8_t* fg,
-                   const uint8_t* bg, int64_t M, int L, void* roi, double* stats, const uint64_t* host_peers,
-                   int n_peers, cudaStream_t st) {
-  const bool with_stats = stats != nullptr;
-  if (itemsize < 2) return MGB_EALIGN;
-  const int unit = itemsize / 2;
-  const int64_t Wu = W * unit;            // logical row length in 16-bit units
-  const int64_t Pu = pitch * unit;        // row pitch in 16-bit units
-  const int wu = L * unit;
-  const int wpu = (wu + 7 + 7) & ~7;            // any shift 0..7 plus the row, in whole vectors
-  if ((Pu * 2) % 16 != 0 || !aligned16(image) || wpu > 256 || L > 256) return MGB_EALIGN;
-  if (C * T > INT32_MAX || H > INT32_MAX || Pu > INT32_MAX || M > INT32_MAX) return MGB_EALIGN;
-  if (with_stats && Tm > 65535) return MGB_EALIGN;
-  PFN_cuTensorMapEncodeTiled encode = get_encode_fn();
-  if (!encode) return MGB_EALIGN;
-
-  TmaGatherParams p{};
-  p.roi = (uint16_t*)roi; p.boxes = boxes; p.order = order; p.mask_t = mask_t; p.fg = fg; p.bg = bg; p.stats = stats;
-  p.C = C; p.T = T; p.Tm = with_stats ? Tm : 1; p.rows = L; p.wu = wu; p.wpu = wpu; p.unit = unit;
-  p.n_peers = 0;
-  if (host_peers && n_peers > 0) {
-    if (n_peers > 8 || !with_stats) return MGB_EINVAL;
-    p.n_peers = n_peers;
-    for (int j = 0; j < n_peers; ++j) p.peer_stats[j] = reinterpret_cast<double*>(host_peers[j]);
-  }
-  p.stage_bytes = (L * wpu * 2 + 127) & ~127;
-  const bool out16 = !roi || aligned16(roi);
-  const bool out4 = !roi || (reinterpret_cast<uintptr_t>(roi) & 3u) == 0;
-  // vpr / half = 1 has no 32-bit multiply-high magic number (ceil(2^32 / 1)): rows of one vector take
-  // the word loop, rows of one word the generic loop
-  if (wu % 8 == 0 && wu > 8 && out16) {
-    p.vpr = (uint32_t)(wu / 8);
-    p.magic_vpr = magic_u32(p.vpr);
-  } else if (wu % 2 == 0 && wu > 2 && out4) {
-    p.half = (uint32_t)(wu / 2);
-    p.magic_half = magic_u32(p.half);
-  }
-  const size_t mask_bytes = with_stats ? 2 * (size_t)((L * wu + 15) & ~15) : 0;
-  const size_t fixed = mask_bytes + kTmaMaxWarps * 8 * sizeof(uint64_t) + (size_t)T * sizeof(int32_t) + 128;
-  int dev = 0, max_smem = 0;
-  MGB_CUDA_TRY(cudaGetDevice(&dev));
-  MGB_CUDA_TRY(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-  const size_t budget = (size_t)max_smem > fixed + 1024 ? (size_t)max_smem - fixed - 1024 : 0;
+int roi_gather_tma(const GatherArgs& a, cudaStream_t st) {
+  if (a.itemsize < 2) return MGB_EALIGN;
+  StagedWindow w;
+  const int rc = stage_window(a, w);
+  if (rc != MGB_OK) return rc;
+  TmaGatherParams& p = w.p;
+  const int64_t M = a.M;
+  const int L = a.L, wu = p.wu;
+  choose_copy_loop(p, a.roi, false);
+  const size_t mask_bytes = a.with_stats ? 2 * (size_t)((L * wu + 15) & ~15) : 0;
+  const size_t fixed = mask_bytes + kTmaMaxWarps * 8 * sizeof(uint64_t) + (size_t)a.T * sizeof(int32_t) + 128;
+  const size_t budget = (size_t)w.max_smem > fixed + 1024 ? (size_t)w.max_smem - fixed - 1024 : 0;
   int nw = kTmaMaxWarps;
   if (const char* e = getenv("MGB_GATHER_WARPS")) nw = atoi(e) == 4 ? 4 : kTmaMaxWarps;   // tuning only
   int ns = (int)(budget / ((size_t)nw * p.stage_bytes));
@@ -447,45 +372,27 @@ int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64
   if (ns < 2) return MGB_EALIGN;
   p.n_stages = ns;
   const size_t smem_bytes = (size_t)nw * ns * p.stage_bytes + fixed;
-
-  CUtensorMap tmap;
-  // the tensor covers the whole pitch: the padding columns are real memory, never needed by a window
-  const cuuint64_t gdim[3] = {(cuuint64_t)Pu, (cuuint64_t)H, (cuuint64_t)(C * T)};
-  const cuuint64_t gstride[2] = {(cuuint64_t)Pu * 2, (cuuint64_t)H * Pu * 2};
-  const cuuint32_t box[3] = {(cuuint32_t)wpu, (cuuint32_t)L, 1};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  const CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 3, const_cast<void*>(image), gdim, gstride, box,
-                             estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                             CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (cr != CUDA_SUCCESS) return MGB_EALIGN;
-
   p.loader = g_gather_loader;
-  p.image = (const uint16_t*)image;
-  p.H = H;
-  p.Wu = Pu;
 
   // Many markers, rows that are not whole 16-byte vectors, few quads per lane: warp-per-marker.
-  const int nquads = (L * wu) / 4;
-  const int qpl = (nquads + 31) / 32;
-  const bool masks_0_1_words = !with_stats || (((size_t)L * L) % 4 == 0 && (reinterpret_cast<uintptr_t>(fg) & 3u) == 0 &&
-                                               (reinterpret_cast<uintptr_t>(bg) & 3u) == 0);
-  const bool out8 = !roi || (reinterpret_cast<uintptr_t>(roi) & 7u) == 0;
-  if (g_gather_wpm && unit == 1 && p.vpr == 0 && wu % 2 == 0 && (L * wu) % 4 == 0 && qpl <= 24 && M >= 2048 &&
-      masks_0_1_words && out8) {
-    const size_t fixed_w = kTmaMaxWarps * 8 * sizeof(uint64_t) + (size_t)T * sizeof(int32_t) + 128;
-    const size_t budget_w = (size_t)max_smem > fixed_w + 1024 ? (size_t)max_smem - fixed_w - 1024 : 0;
+  const int qpl = ((L * wu) / 4 + 31) / 32;
+  const bool masks_0_1_words = !a.with_stats || (((size_t)L * L) % 4 == 0 && (reinterpret_cast<uintptr_t>(a.fg) & 3u) == 0 &&
+                                                 (reinterpret_cast<uintptr_t>(a.bg) & 3u) == 0);
+  if (g_gather_wpm && p.unit == 1 && copy_loop(L, wu, a.roi, true) == CopyLoop::kQuad && M >= 2048 && masks_0_1_words) {
+    const size_t fixed_w = kTmaMaxWarps * 8 * sizeof(uint64_t) + (size_t)a.T * sizeof(int32_t) + 128;
+    const size_t budget_w = (size_t)w.max_smem > fixed_w + 1024 ? (size_t)w.max_smem - fixed_w - 1024 : 0;
     int ns_w = (int)(budget_w / ((size_t)kTmaMaxWarps * p.stage_bytes));
     if (ns_w > 4) ns_w = 4;
     if (ns_w >= 2) {
       TmaGatherParams pw = p;
       pw.n_stages = ns_w;
       const size_t smem_w = (size_t)kTmaMaxWarps * ns_w * p.stage_bytes + fixed_w;
-      dim3 grid_w((unsigned)((M + kTmaMaxWarps - 1) / kTmaMaxWarps), (unsigned)(with_stats ? Tm : 1));
+      dim3 grid_w((unsigned)((M + kTmaMaxWarps - 1) / kTmaMaxWarps), (unsigned)p.Tm);
 #define MGB_LAUNCH_W(ST, SO, QP)                                                                       \
   do {                                                                                                 \
     MGB_CUDA_TRY(cudaFuncSetAttribute(roi_gather_wpm_kernel<ST, SO, QP>,                               \
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));      \
-    roi_gather_wpm_kernel<ST, SO, QP><<<grid_w, kTmaMaxWarps * 32, smem_w, st>>>(tmap, pw, M);         \
+    roi_gather_wpm_kernel<ST, SO, QP><<<grid_w, kTmaMaxWarps * 32, smem_w, st>>>(w.tmap, pw, M);       \
   } while (0)
 #define MGB_LAUNCH_WQ(ST, SO)                      \
   do {                                             \
@@ -493,8 +400,8 @@ int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64
     else if (qpl <= 20) MGB_LAUNCH_W(ST, SO, 20);  \
     else MGB_LAUNCH_W(ST, SO, 24);                 \
   } while (0)
-      if (with_stats) {
-        if (roi) MGB_LAUNCH_WQ(true, true);
+      if (a.with_stats) {
+        if (a.roi) MGB_LAUNCH_WQ(true, true);
         else MGB_LAUNCH_WQ(true, false);
       } else {
         MGB_LAUNCH_WQ(false, true);
@@ -506,12 +413,12 @@ int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64
     }
   }
   const int vpl = p.vpr ? (int)((L * p.vpr + 31) / 32) : 0;       // vectors per lane
-  dim3 grid((unsigned)M, (unsigned)(with_stats ? Tm : 1));
+  dim3 grid((unsigned)M, (unsigned)p.Tm);
 #define MGB_LAUNCH(ST, SO, VP)                                                                          \
   do {                                                                                                  \
     MGB_CUDA_TRY(cudaFuncSetAttribute(roi_gather_tma_kernel<ST, SO, VP>,                                \
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));   \
-    roi_gather_tma_kernel<ST, SO, VP><<<grid, nw * 32, smem_bytes, st>>>(tmap, p);                      \
+    roi_gather_tma_kernel<ST, SO, VP><<<grid, nw * 32, smem_bytes, st>>>(w.tmap, p);                    \
   } while (0)
 #define MGB_LAUNCH_V(ST, SO)                                  \
   do {                                                        \
@@ -520,8 +427,8 @@ int roi_gather_tma(const void* image, int64_t pitch, int64_t C, int64_t T, int64
     else if (vpl > 21 && vpl <= 36) MGB_LAUNCH(ST, SO, 36);   \
     else MGB_LAUNCH(ST, SO, 0);                               \
   } while (0)
-  if (with_stats) {
-    if (roi) MGB_LAUNCH_V(true, true);
+  if (a.with_stats) {
+    if (a.roi) MGB_LAUNCH_V(true, true);
     else MGB_LAUNCH_V(true, false);
   } else {
     MGB_LAUNCH_V(false, true);
