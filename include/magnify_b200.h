@@ -144,6 +144,13 @@ int mgb_set_tma_enabled(int enabled);
  * kernel that otherwise handles many-marker / few-window shapes (bead screens).  Returns the
  * previous value; results do not depend on it. */
 int mgb_set_gather_loader(int loader);
+/* Diagnostic: which kernel the last ROI-gather launch of this process used (host memory, no device
+ * access).  host_out[0..8] = kernel (1 lists-CTA, 2 lists-WPM, 3 staged-CTA, 4 staged-WPM,
+ * 5 plain-words, 6 plain-scalar), unrolled vectors / quads per lane (0: run-time loop), copy loop
+ * (0 vector, 1 quad, 2 word, 3 element), warps per CTA, stages per warp (0: not staged), loader
+ * (0 TMA, 1 cp.async, -1 not staged), summaries (0/1), crops stored (0/1), and the keys per thread of
+ * the last exact-median launch (0: the kernel for L > 160).  -1 where nothing has run yet. */
+int mgb_last_gather_path(int32_t* host_out);
 
 /* ---- F4 (+R): ROI gather, reference find.py:160-169, 324-334, 370-377, 589-602 -------------
  * roi[m,c,t] = image[c,t, top:top+L, left:left+L] for any itemsize in {1,2,4,8}.
@@ -205,7 +212,9 @@ int mgb_roi_median_u16(const uint16_t* roi, int64_t M, int64_t C, int64_t T, int
 
 /* The same two reductions for a float32 roi (the reference accepts float images, tests/test_chip.py:76-96):
  * float64 accumulation in a fixed order, NaN pixels skipped (nanmean / nanmedian); the median is the
- * exact middle value (mean of the two middle values for even counts) as float64. */
+ * exact middle value, or for even counts the mean of the two middle values computed in float32 as
+ * np.nanmedian does for a float32 array (sum rounded to float32, inf on overflow, then halved),
+ * returned as float64. */
 int mgb_roi_stats_f32(const float* roi, int64_t M, int64_t C, int64_t T, int L, const int32_t* mask_t, int64_t Tm,
                       const uint8_t* fg, const uint8_t* bg, double* stats, void* stream);
 int mgb_roi_median_f32(const float* roi, int64_t M, int64_t C, int64_t T, int L, const int32_t* mask_t, int64_t Tm,

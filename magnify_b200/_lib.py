@@ -34,6 +34,7 @@ SIGNATURES = {
     "mgb_set_tma_enabled": [c_int],
     "mgb_set_stitch_variant": [c_int],
     "mgb_set_gather_loader": [c_int],
+    "mgb_last_gather_path": [POINTER(ctypes.c_int32)],
     "mgb_stitch": [_P, _P, _I64, _I64, _I64, _I64, _I64, _I64, _I64, _I64, c_int, POINTER(c_int), _P],
     "mgb_flatfield_tilemax_u16": [_P, _I64, _I64, _I64, c_int, c_int, _P, _P],
     "mgb_flatfield_maxima": [_P, c_int, c_int, _I64, _P, _P, _P, _P],

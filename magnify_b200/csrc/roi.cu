@@ -198,6 +198,19 @@ template <> __device__ __forceinline__ double median_value<uint16_t>(uint32_t ke
 template <> __device__ __forceinline__ double median_value<float>(uint32_t key) {
   return (double)__uint_as_float((key & 0x80000000u) ? (key & 0x7fffffffu) : ~key);
 }
+// The median from the two middle keys (equal for an odd count), computed in the dtype the reference
+// reduces in: `roi.where(mask)` keeps a float32 roi float32, and np.nanmedian then averages the two
+// middle values in float32 -- the sum rounded once (inf where it overflows), then halved.  uint16
+// values and the half of their sum are exact in any float type.
+template <typename TPix> __device__ __forceinline__ double median_mid(uint32_t k1, uint32_t k2, bool even);
+template <> __device__ __forceinline__ double median_mid<uint16_t>(uint32_t k1, uint32_t k2, bool) {
+  return 0.5 * (median_value<uint16_t>(k1) + median_value<uint16_t>(k2));
+}
+template <> __device__ __forceinline__ double median_mid<float>(uint32_t k1, uint32_t k2, bool even) {
+  const float a = (float)median_value<float>(k1);
+  if (!even) return (double)a;
+  return (double)__fmul_rn(__fadd_rn(a, (float)median_value<float>(k2)), 0.5f);
+}
 
 // One CTA per ROI.  Every thread keeps its pixels as 32-bit keys (masked-out -> 0xffffffff) in
 // registers; the k-th smallest is found by a binary search on the key with one block count per
@@ -288,7 +301,7 @@ roi_median_kernel(const TPix* __restrict__ roi, int64_t C, int64_t T, int L,
     for (int i = 0; i < kThreads / 32; ++i) g = min(g, red[buf][i]);
     if (tot < k1 + 2) v2 = g;
   }
-  if (threadIdx.x == 0) median[n * stride] = 0.5 * (median_value<TPix>(v1) + median_value<TPix>(v2));
+  if (threadIdx.x == 0) median[n * stride] = median_mid<TPix>(v1, v2, (nvalid & 1u) == 0);
 }
 
 // Any L: the keys do not fit in registers, so every bisection step re-reads the window (it stays
@@ -345,7 +358,7 @@ roi_median_big_kernel(const TPix* __restrict__ roi, int64_t C, int64_t T, int L,
     sweep(lo, &cnt, &above, &dummy);
     if (cnt < k1 + 2) v2 = above;
   }
-  if (threadIdx.x == 0) median[n * stride] = 0.5 * (median_value<TPix>(lo) + median_value<TPix>(v2));
+  if (threadIdx.x == 0) median[n * stride] = median_mid<TPix>(lo, v2, (nvalid & 1u) == 0);
 }
 
 // Masked sums of a float32 roi: one CTA per (m, c, t), float64 accumulation in a fixed order
@@ -389,6 +402,16 @@ roi_stats_f32_kernel(const float* __restrict__ roi, int64_t C, int64_t T, int L,
 
 static int g_tma_enabled = 1;
 
+// mgb_last_gather_path's record: kernel, unroll, copy loop, warps, stages, loader, stats, store,
+// median keys per thread (0: the big-window kernel); -1 until the first launch.
+static int32_t g_last_path[9] = {-1, -1, -1, -1, -1, -1, -1, -1, -1};
+
+void record_gather_path(GatherKernel kernel, int unroll, CopyLoop loop, int warps, int stages, int loader,
+                        bool stats, bool store) {
+  const int32_t v[8] = {kernel, unroll, (int32_t)loop, warps, stages, loader, stats, store};
+  for (int i = 0; i < 8; ++i) g_last_path[i] = v[i];
+}
+
 }  // namespace mgb
 
 using namespace mgb;
@@ -403,14 +426,21 @@ static int launch_roi_median(const TPix* roi, int64_t M, int64_t C, int64_t T, i
   if (!roi || !mask_t || !mask || !median || Tm <= 0) return MGB_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   const int npt = (int)ceil_div((int64_t)L * L, kThreads);
-#define MGB_MED(N) roi_median_kernel<N, TPix><<<(unsigned)n_roi, kThreads, 0, st>>>(roi, C, T, L, mask_t, Tm, mask, median, stride)
+#define MGB_MED(N)                                                                                              \
+  do {                                                                                                          \
+    roi_median_kernel<N, TPix><<<(unsigned)n_roi, kThreads, 0, st>>>(roi, C, T, L, mask_t, Tm, mask, median, stride); \
+    g_last_path[8] = N;                                                                                         \
+  } while (0)
   if (npt <= 4) MGB_MED(4);
   else if (npt <= 10) MGB_MED(10);
   else if (npt <= 21) MGB_MED(21);
   else if (npt <= 40) MGB_MED(40);
   else if (npt <= 64) MGB_MED(64);
   else if (npt <= 100) MGB_MED(100);
-  else roi_median_big_kernel<TPix><<<(unsigned)n_roi, kThreads, 0, st>>>(roi, C, T, L, mask_t, Tm, mask, median, stride);   // L > 160
+  else {   // L > 160
+    roi_median_big_kernel<TPix><<<(unsigned)n_roi, kThreads, 0, st>>>(roi, C, T, L, mask_t, Tm, mask, median, stride);
+    g_last_path[8] = 0;
+  }
 #undef MGB_MED
   MGB_CUDA_LAUNCH_CHECK();
   return MGB_OK;
@@ -470,10 +500,12 @@ static int gather_common(const GatherArgs& a, cudaStream_t st, int* host_median_
     p.mask_t = a.mask_t; p.Tm = a.Tm; p.fg = a.fg; p.bg = a.bg; p.stats = a.stats;
     if (a.with_stats) roi_gather_words_kernel<true><<<(unsigned)n_roi, kThreads, 0, st>>>(p);
     else roi_gather_words_kernel<false><<<(unsigned)n_roi, kThreads, 0, st>>>(p);
+    record_gather_path(kGatherPlainWords, 0, CopyLoop::kWord, kThreads / 32, 0, -1, a.with_stats, a.roi);
   } else if (a.with_stats) {
     roi_gather_scalar_kernel<uint16_t, true><<<(unsigned)n_roi, kThreads, 0, st>>>(
         (const uint16_t*)a.image, (uint16_t*)a.roi, C, T, H, pitch, a.boxes, a.marker_stride, L, a.mask_t, a.Tm, a.fg,
         a.bg, a.stats);
+    record_gather_path(kGatherPlainScalar, 0, CopyLoop::kElement, kThreads / 32, 0, -1, true, a.roi);
   } else {
     const int32_t* boxes = a.boxes;
     const int64_t ms = a.marker_stride;
@@ -483,6 +515,7 @@ static int gather_common(const GatherArgs& a, cudaStream_t st, int* host_median_
       case 4: roi_gather_scalar_kernel<uint32_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint32_t*)a.image, (uint32_t*)a.roi, C, T, H, pitch, boxes, ms, L, nullptr, 0, nullptr, nullptr, nullptr); break;
       default: roi_gather_scalar_kernel<uint64_t, false><<<(unsigned)n_roi, kThreads, 0, st>>>((const uint64_t*)a.image, (uint64_t*)a.roi, C, T, H, pitch, boxes, ms, L, nullptr, 0, nullptr, nullptr, nullptr); break;
     }
+    record_gather_path(kGatherPlainScalar, 0, CopyLoop::kElement, kThreads / 32, 0, -1, false, true);
   }
   MGB_CUDA_LAUNCH_CHECK();
   return MGB_OK;
@@ -492,6 +525,12 @@ int mgb_set_tma_enabled(int enabled) {
   const int old = g_tma_enabled;
   g_tma_enabled = enabled ? 1 : 0;
   return old;
+}
+
+int mgb_last_gather_path(int32_t* host_out) {
+  if (!host_out) return MGB_EINVAL;
+  for (int i = 0; i < 9; ++i) host_out[i] = g_last_path[i];
+  return MGB_OK;
 }
 
 int mgb_set_gather_loader(int loader) {

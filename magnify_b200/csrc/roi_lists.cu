@@ -580,6 +580,7 @@ int roi_gather_lists(const GatherArgs& a, cudaStream_t st) {
       }                                                                                                   \
     }                                                                                                     \
     kern<<<grid, nw * 32, smem_bytes, st>>>(w.tmap, p, M, magic_l);                                       \
+    record_gather_path(WP ? kGatherListsWpm : kGatherListsCta, VP ? VP : QP, loop, nw, ns, 0, true, a.roi);  \
   } while (0)
 #define MGB_LAUNCH_NW(VP, QP, WP)                       \
   do {                                                  \

@@ -384,4 +384,11 @@ inline CopyLoop choose_copy_loop(TmaGatherParams& p, const void* roi, bool quads
   return loop;
 }
 
+// Host-side record of the last gather launch, read back by mgb_last_gather_path (a diagnostic:
+// the launchers write it next to each launch, no kernel reads it).
+enum GatherKernel { kGatherListsCta = 1, kGatherListsWpm, kGatherStagedCta, kGatherStagedWpm,
+                    kGatherPlainWords, kGatherPlainScalar };
+void record_gather_path(GatherKernel kernel, int unroll, CopyLoop loop, int warps, int stages, int loader,
+                        bool stats, bool store);   // roi.cu
+
 }  // namespace mgb

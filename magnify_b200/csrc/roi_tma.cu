@@ -357,7 +357,7 @@ int roi_gather_tma(const GatherArgs& a, cudaStream_t st) {
   TmaGatherParams& p = w.p;
   const int64_t M = a.M;
   const int L = a.L, wu = p.wu;
-  choose_copy_loop(p, a.roi, false);
+  const CopyLoop loop = choose_copy_loop(p, a.roi, false);
   const size_t mask_bytes = a.with_stats ? 2 * (size_t)((L * wu + 15) & ~15) : 0;
   const size_t fixed = mask_bytes + kTmaMaxWarps * 8 * sizeof(uint64_t) + (size_t)a.T * sizeof(int32_t) + 128;
   const size_t budget = (size_t)w.max_smem > fixed + 1024 ? (size_t)w.max_smem - fixed - 1024 : 0;
@@ -393,6 +393,7 @@ int roi_gather_tma(const GatherArgs& a, cudaStream_t st) {
     MGB_CUDA_TRY(cudaFuncSetAttribute(roi_gather_wpm_kernel<ST, SO, QP>,                               \
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));      \
     roi_gather_wpm_kernel<ST, SO, QP><<<grid_w, kTmaMaxWarps * 32, smem_w, st>>>(w.tmap, pw, M);       \
+    record_gather_path(kGatherStagedWpm, QP, CopyLoop::kQuad, kTmaMaxWarps, ns_w, 0, ST, SO);           \
   } while (0)
 #define MGB_LAUNCH_WQ(ST, SO)                      \
   do {                                             \
@@ -419,6 +420,7 @@ int roi_gather_tma(const GatherArgs& a, cudaStream_t st) {
     MGB_CUDA_TRY(cudaFuncSetAttribute(roi_gather_tma_kernel<ST, SO, VP>,                                \
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));   \
     roi_gather_tma_kernel<ST, SO, VP><<<grid, nw * 32, smem_bytes, st>>>(w.tmap, p);                    \
+    record_gather_path(kGatherStagedCta, VP, loop, nw, ns, p.loader, ST, SO);                           \
   } while (0)
 #define MGB_LAUNCH_V(ST, SO)                                  \
   do {                                                        \

@@ -12,6 +12,7 @@ Layouts follow the reference (see SURVEY.md section 8a):
 from __future__ import annotations
 
 import ctypes
+from collections import namedtuple
 from typing import Optional, Sequence
 
 import numpy as np
@@ -456,6 +457,26 @@ def mask_count_max(fg: torch.Tensor, bg: torch.Tensor):
 
 
 last_gather_fused = True   # diagnostic: did the last roi_gather_stats call get its medians from the fused kernel?
+
+GatherPath = namedtuple("GatherPath", "kernel unroll copy_loop warps stages loader stats store median_npt")
+_GATHER_KERNELS = {1: "lists-cta", 2: "lists-wpm", 3: "staged-cta", 4: "staged-wpm", 5: "plain-words",
+                   6: "plain-scalar"}
+_COPY_LOOPS = {0: "vector", 1: "quad", 2: "word", 3: "element"}
+_LOADERS = {0: "tma", 1: "cp.async"}
+
+
+def last_gather_path() -> GatherPath:
+    """Diagnostic: the kernel the last ROI-gather launch of this process ran (`roi_gather`,
+    `roi_gather_stats`, `roi_stats` of a uint16 roi) and its compiled configuration -- vectors or
+    quads per lane `unroll` (0: run-time loop), `copy_loop`, warps per CTA, stages per warp (0: not
+    staged), `loader` (None: not staged), whether it summed and stored crops -- plus the keys per
+    thread of the last exact-median launch (`median_npt`, 0: the kernel for L > 160).  Read from
+    host memory: no synchronisation.  Fields are None where nothing has run yet."""
+    raw = (ctypes.c_int32 * 9)()
+    _lib.call("mgb_last_gather_path", raw)
+    v = [None if x < 0 else int(x) for x in raw]
+    return GatherPath(_GATHER_KERNELS.get(v[0]), v[1], _COPY_LOOPS.get(v[2]), v[3], v[4], _LOADERS.get(v[5]),
+                      None if v[6] is None else bool(v[6]), None if v[7] is None else bool(v[7]), v[8])
 
 
 def roi_gather_stats(

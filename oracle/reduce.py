@@ -5,13 +5,24 @@ test asserts an intensity).  The reference expressions are xarray's
 `roi.where(fg).mean(dim=["roi_x","roi_y"])` / `.median(...)` / `fg.sum(...)`
 (src/magnify/identify.py:76-80, filter.py:21-22,51,74,82, README.md:21-22): `where` fills
 masked-out pixels with NaN and the reductions skip NaN (nanmean / nanmedian), so an empty
-mask yields NaN.  Restated here in float64.
+mask yields NaN.  Restated here in float64, except the medians of a float roi: `where` keeps a
+float32 roi float32, and np.nanmedian averages the two middle values of a float32 array in float32
+(the sum rounded to float32, inf where it overflows, then halved).  Integer rois are widened by
+`where`; the half-sum of two 16-bit values is exact in any float type, so their medians are taken
+in float64.  (For fewer than 600 pixels per window np.nanmedian takes a masked-array path that also
+"averages" an odd count's single middle value with itself, so a float32 middle value above half the
+float32 maximum becomes inf there; the kernels return the middle value, as np.median does.)
 """
 from __future__ import annotations
 
 import warnings
 
 import numpy as np
+
+def _median_values(roi: np.ndarray) -> np.ndarray:
+    """roi in the dtype `roi.where(mask)` reduces its median in (see the module docstring)."""
+    return roi if np.issubdtype(roi.dtype, np.floating) else roi.astype(np.float64)
+
 
 STATS = ("n_fg", "n_bg", "sum_fg", "sum_bg", "mean_fg", "mean_bg", "median_fg", "median_bg")
 
@@ -21,6 +32,7 @@ def masked_stats(roi: np.ndarray, fg: np.ndarray, bg: np.ndarray) -> np.ndarray:
     m, c, t = roi.shape[:3]
     out = np.empty((m, c, t, len(STATS)), dtype=np.float64)
     r = roi.astype(np.float64)
+    rm = _median_values(roi)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore", RuntimeWarning)
         for k, mask in enumerate((fg, bg)):
@@ -29,18 +41,19 @@ def masked_stats(roi: np.ndarray, fg: np.ndarray, bg: np.ndarray) -> np.ndarray:
             out[..., 0 + k] = np.broadcast_to(mask.sum(axis=(-2, -1))[:, None], (m, c, t))
             out[..., 2 + k] = np.nansum(vals, axis=(-2, -1))
             out[..., 4 + k] = np.nanmean(vals, axis=(-2, -1))
-            out[..., 6 + k] = np.nanmedian(vals.reshape(vals.shape[:3] + (-1,)), axis=-1)
+            med = np.where(mk, rm, rm.dtype.type(np.nan))
+            out[..., 6 + k] = np.nanmedian(med.reshape(med.shape[:3] + (-1,)), axis=-1)
     return out
 
 
 def masked_median(roi: np.ndarray, mask: np.ndarray) -> np.ndarray:
     """`roi.where(mask).median(dim=["roi_x","roi_y"])` -> (M, C, T) float64 (NaN when empty)."""
-    r = roi.astype(np.float64)
-    vals = np.where(np.broadcast_to(mask[:, None], r.shape), r, np.nan)
+    r = _median_values(roi)
+    vals = np.where(np.broadcast_to(mask[:, None], r.shape), r, r.dtype.type(np.nan))
     flat = vals.reshape(vals.shape[:3] + (-1,))
     with warnings.catch_warnings():
         warnings.simplefilter("ignore", RuntimeWarning)
-        return np.nanmedian(flat, axis=-1)
+        return np.nanmedian(flat, axis=-1).astype(np.float64)
 
 
 def mrbles_intensities(roi: np.ndarray, fg: np.ndarray, bg: np.ndarray) -> np.ndarray:

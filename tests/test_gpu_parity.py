@@ -616,10 +616,11 @@ def test_random_gather_sweep(cuda_device):
         np.testing.assert_array_equal(med, o_red.masked_median(want_roi, fg[:, mask_t]), err_msg=msg)
 
 
-def test_float32_roi_stats_and_median(cuda_device):
+def test_float32_roi_stats_and_float32_median(cuda_device):
     """The reductions on a float32 roi (the reference accepts float images): float64 sums in a
-    fixed order (rtol 1e-12 against NumPy's float64 sums), exact medians, NaN pixels and empty
-    masks handled like nanmean / nanmedian."""
+    fixed order (rtol 1e-12 against NumPy's float64 sums), exact medians (the two middle values
+    of an even count averaged in float32, like np.nanmedian of the float32 roi), NaN pixels and
+    empty masks handled like nanmean / nanmedian."""
     from magnify_b200 import ops
 
     rng = np.random.default_rng(31)
@@ -648,12 +649,16 @@ def test_float32_roi_stats_and_median(cuda_device):
                     with np.errstate(invalid="ignore", divide="ignore"):
                         means = [np.float64(want[2]) / want[0], np.float64(want[3]) / want[1]]
                     np.testing.assert_allclose(stats[mi, ci, ti, 4:6], means, rtol=1e-12, equal_nan=True)
-                    vals = np.sort(px[f & ok])
+                    vals = np.sort(roi[mi, ci, ti][f & ok])
                     if len(vals) == 0:
                         assert np.isnan(med[mi, ci, ti]) and np.isnan(stats[mi, ci, ti, 6])
                     else:
+                        # `where` keeps the float32 roi float32: the two middle values are averaged
+                        # in float32, as np.nanmedian does
                         lo, hi = vals[(len(vals) - 1) // 2], vals[len(vals) // 2]
-                        assert med[mi, ci, ti] == 0.5 * (lo + hi), (length, mi, ci, ti)
+                        want_med = np.float64(lo if len(vals) % 2 else (lo + hi) / np.float32(2))
+                        assert want_med == np.float64(np.median(vals)), (length, mi, ci, ti)
+                        assert med[mi, ci, ti] == want_med, (length, mi, ci, ti)
                         assert stats[mi, ci, ti, 6] == med[mi, ci, ti]
 
 
