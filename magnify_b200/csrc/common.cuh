@@ -87,4 +87,31 @@ __device__ __forceinline__ void atomic_max_nonneg_f64(double* addr, double v) {
             static_cast<unsigned long long>(__double_as_longlong(v)));
 }
 
+__device__ __forceinline__ double nan_f64() { return __longlong_as_double(0x7ff8000000000000LL); }
+
+// 8 consecutive 16-bit units starting S units into the 16 units of (a, b).
+template <int S>
+__device__ __forceinline__ uint4 shift_units(const uint4& a, const uint4& b) {
+  const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+  constexpr int o = S >> 1;
+  if constexpr ((S & 1) == 0) {
+    return make_uint4(w[o], w[o + 1], w[o + 2], w[o + 3]);
+  } else {
+    return make_uint4(__funnelshift_r(w[o], w[o + 1], 16), __funnelshift_r(w[o + 1], w[o + 2], 16),
+                      __funnelshift_r(w[o + 2], w[o + 3], 16), __funnelshift_r(w[o + 3], w[o + 4], 16));
+  }
+}
+
+// 16-byte global -> shared copy that bypasses L1 (cp.async.cg, SASS LDGSTS), and its completion:
+// commit closes a group of copies, wait<N> returns once at most N groups are still in flight.
+__device__ __forceinline__ void cp_async16(uint32_t smem_addr, const void* gptr) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() {
+  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
 }  // namespace mgb

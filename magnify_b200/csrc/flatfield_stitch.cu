@@ -67,24 +67,20 @@ __device__ __forceinline__ double block_max(double v, double* smem) {
   return v;
 }
 
-__global__ void __launch_bounds__(kThreads)
-ff_maxima_kernel(const uint16_t* __restrict__ xmax_partial, int splits, int K, int64_t HW,
-                 const double* __restrict__ flat, const double* __restrict__ dark,
-                 double* __restrict__ maxima) {
+// One pixel: t = max(x - dark, 0) and u = t / flat in the reference's operation order, folded into
+// the running maxima m1 of t and m2 of u.  xarray's max skips NaN (preprocess.py:84,86); fmax does
+// the same.
+__device__ __forceinline__ void ff_maxima_step(double x, double dark, double flat, double& m1, double& m2) {
+  double t = __dsub_rn(x, dark);
+  t = t < 0.0 ? 0.0 : t;
+  const double u = __ddiv_rn(t, flat);
+  m1 = fmax(m1, t);
+  m2 = fmax(m2, u);
+}
+
+// The block's maxima folded into maxima[0] (t) and maxima[1] (u).
+__device__ __forceinline__ void ff_maxima_finish(double m1, double m2, double* maxima) {
   __shared__ double sm[2][kThreads / 32];
-  double m1 = 0.0, m2 = 0.0;
-  const int64_t total = (int64_t)K * HW;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
-       i += (int64_t)gridDim.x * blockDim.x) {
-    unsigned x = 0;
-    for (int s = 0; s < splits; ++s) x = max(x, (unsigned)xmax_partial[(int64_t)s * total + i]);
-    double t = __dsub_rn((double)x, dark[i]);
-    t = t < 0.0 ? 0.0 : t;
-    double u = __ddiv_rn(t, flat[i]);
-    // xarray's max skips NaN (preprocess.py:84,86); fmax does the same.
-    m1 = fmax(m1, t);
-    m2 = fmax(m2, u);
-  }
   m1 = block_max(m1, sm[0]);
   m2 = block_max(m2, sm[1]);
   if (threadIdx.x == 0) {
@@ -93,30 +89,35 @@ ff_maxima_kernel(const uint16_t* __restrict__ xmax_partial, int splits, int K, i
   }
 }
 
+__global__ void __launch_bounds__(kThreads)
+ff_maxima_kernel(const uint16_t* __restrict__ xmax_partial, int splits, int K, int64_t HW,
+                 const double* __restrict__ flat, const double* __restrict__ dark,
+                 double* __restrict__ maxima) {
+  double m1 = 0.0, m2 = 0.0;
+  const int64_t total = (int64_t)K * HW;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    unsigned x = 0;
+    for (int s = 0; s < splits; ++s) x = max(x, (unsigned)xmax_partial[(int64_t)s * total + i]);
+    ff_maxima_step((double)x, dark[i], flat[i], m1, m2);
+  }
+  ff_maxima_finish(m1, m2, maxima);
+}
+
 template <typename T>
 __global__ void __launch_bounds__(kThreads)
 ff_maxima_generic_kernel(const T* __restrict__ tiles, int64_t C, int64_t P, int64_t HW, int K,
                          const double* __restrict__ flat, const double* __restrict__ dark,
                          double* __restrict__ maxima) {
-  __shared__ double sm[2][kThreads / 32];
   double m1 = 0.0, m2 = 0.0;
   const int64_t total = C * P * HW;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t pos = i % HW;
     const int64_t k = (K == 1) ? 0 : i / (P * HW);
-    double t = __dsub_rn((double)tiles[i], dark[k * HW + pos]);
-    t = t < 0.0 ? 0.0 : t;
-    double u = __ddiv_rn(t, flat[k * HW + pos]);
-    m1 = fmax(m1, t);
-    m2 = fmax(m2, u);
+    ff_maxima_step((double)tiles[i], dark[k * HW + pos], flat[k * HW + pos], m1, m2);
   }
-  m1 = block_max(m1, sm[0]);
-  m2 = block_max(m2, sm[1]);
-  if (threadIdx.x == 0) {
-    atomic_max_nonneg_f64(&maxima[0], m1);
-    atomic_max_nonneg_f64(&maxima[1], m2);
-  }
+  ff_maxima_finish(m1, m2, maxima);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -167,35 +168,12 @@ struct StitchParams {
   const double* maxima;
 };
 
-template <int S>
-__device__ __forceinline__ uint4 funnel8(const uint4& a, const uint4& b) {
-  // 8 consecutive 16-bit units starting S units into the 16 units of (a, b).
-  const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-  constexpr int o = S >> 1;
-  if constexpr ((S & 1) == 0) {
-    return make_uint4(w[o], w[o + 1], w[o + 2], w[o + 3]);
-  } else {
-    return make_uint4(__funnelshift_r(w[o], w[o + 1], 16), __funnelshift_r(w[o + 1], w[o + 2], 16),
-                      __funnelshift_r(w[o + 2], w[o + 3], 16),
-                      __funnelshift_r(w[o + 3], w[o + 4], 16));
-  }
-}
-
 // Prefetch ring: every thread streams its own aligned 16-byte input chunk of the next
 // kStitchStages tiles into shared memory with cp.async (LDGSTS, L1 bypass), so the bytes in
 // flight per SM are decoupled from the register file, which holds the 16 float64 coefficients.
 // A thread reads back its own slot and (for a shifted vector) its right neighbour's, which
 // needs only warp-level synchronisation; every input byte is requested from L2 once.
 constexpr int stitch_smem_bytes(int stages) { return stages * (kThreads + kThreads / 32) * 16; }
-
-__device__ __forceinline__ void cp_async16(uint32_t smem_addr, const void* gptr) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
 
 template <int MODE, int S, int kStitchStages>
 __device__ __forceinline__ void stitch_u16_body(const StitchParams& p, uint4* ring, int q, int k, int split) {
@@ -303,7 +281,7 @@ __device__ __forceinline__ void stitch_u16_body(const StitchParams& p, uint4* ri
     const uint4 vb = (S != 0) ? slot_b[stage * kStageVecs] : va;
     if (++stage == kStitchStages) stage = 0;
 
-    uint4 v = funnel8<S>(va, vb);
+    uint4 v = shift_units<S>(va, vb);
     if constexpr (MODE == 1) {
       const uint32_t win[4] = {v.x, v.y, v.z, v.w};
       uint32_t wout[4];
@@ -482,6 +460,39 @@ static int run_stitch_fast(StitchParams p, cudaStream_t st) {
   return launch_stitch_fast<MODE>(p, st);
 }
 
+// The checks both stitch entry points make, and the geometry of p in 16-bit units (`units` per
+// element along x; rows stay in elements).  An empty stack returns MGB_OK with p->CT == 0: nothing
+// to launch.  K (tables) counts toward the size limits, tables_ok (no table pointer is null) toward
+// the pointer check.  limits_first puts the size limits before the empty-stack shortcut and the
+// null pointers (mgb_stitch), else after them (mgb_flatfield_stitch_u16): an empty stack of too tall
+// tiles is MGB_EUNSUPPORTED for one entry point and MGB_OK for the other.
+static int stitch_setup(const void* tiles, void* image, int64_t image_pitch, int64_t C, int64_t T, int64_t R,
+                        int64_t Cc, int64_t H, int64_t W, int64_t overlap, int units, int K, bool tables_ok,
+                        bool limits_first, StitchParams* p) {
+  *p = StitchParams{};
+  if (C < 0 || T < 0 || R < 0 || Cc < 0 || H <= 0 || W <= 0) return MGB_EINVAL;
+  if (overlap < 0 || overlap >= H || overlap >= W) return MGB_EINVAL;  // stitch.py:8-9,16-20
+  const bool too_large = H > INT32_MAX / 8 || W > INT32_MAX / 8 || R > INT32_MAX || Cc > INT32_MAX || K > 65535;
+  if (limits_first && too_large) return MGB_EUNSUPPORTED;
+  if (C * T == 0 || R == 0 || Cc == 0) return MGB_OK;
+  if (!tiles || !image || !tables_ok) return MGB_EINVAL;
+  if (too_large) return MGB_EUNSUPPORTED;
+  const int clip = (int)(overlap / 2);
+  const int h = (int)(H - overlap), w = (int)(W - overlap);
+  const int64_t pitch = image_pitch > 0 ? image_pitch : Cc * w;
+  if (pitch < Cc * w) return MGB_EINVAL;
+  p->tiles = (const uint16_t*)tiles; p->image = (uint16_t*)image;
+  p->CT = C * T; p->T = (int)T; p->R = (int)R; p->Cc = (int)Cc;
+  p->H = (int)H; p->W = (int)(W * units); p->clip = clip * units; p->clip_y = clip; p->h = h; p->w = w * units;
+  p->Wim = pitch * units; p->Him = R * h; p->K = K;
+  return MGB_OK;
+}
+
+// The vectorised kernels read and write whole 16-byte vectors.
+static bool stitch_vectorisable(const StitchParams& p) {
+  return p.W % 8 == 0 && p.Wim % 8 == 0 && aligned16(p.tiles) && aligned16(p.image);
+}
+
 static int grid_for(int64_t n) {
   int64_t b = ceil_div(n, kThreads);
   const int64_t cap = (int64_t)cached_sm_count() * 32;
@@ -508,38 +519,28 @@ int mgb_stitch(const void* tiles, void* image, int64_t image_pitch, int64_t C, i
                int64_t Cc, int64_t H, int64_t W, int64_t overlap, int itemsize, int* host_used_fast,
                void* stream) {
   if (host_used_fast) *host_used_fast = 0;
-  if (C < 0 || T < 0 || R < 0 || Cc < 0 || H <= 0 || W <= 0) return MGB_EINVAL;
-  if (overlap < 0 || overlap >= H || overlap >= W) return MGB_EINVAL;  // stitch.py:8-9,16-20
   if (itemsize != 1 && itemsize != 2 && itemsize != 4 && itemsize != 8) return MGB_EINVAL;
-  if (H > INT32_MAX / 8 || W > INT32_MAX / 8 || R > INT32_MAX || Cc > INT32_MAX) return MGB_EUNSUPPORTED;
-  const int64_t CT = C * T;
-  const int clip = (int)(overlap / 2);
-  const int h = (int)(H - overlap), w = (int)(W - overlap);
-  if (CT == 0 || R == 0 || Cc == 0) return MGB_OK;
-  if (!tiles || !image) return MGB_EINVAL;
+  // 16-bit units per element; bytes (element-wise kernel only) keep the geometry in elements
+  const int u = itemsize >= 2 ? itemsize / 2 : 1;
+  StitchParams p;
+  const int rc = stitch_setup(tiles, image, image_pitch, C, T, R, Cc, H, W, overlap, u, /*K=*/1,
+                              /*tables_ok=*/true, /*limits_first=*/true, &p);
+  if (rc != MGB_OK || p.CT == 0) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  const int64_t Wim = Cc * w;
-  const int64_t pitch = image_pitch > 0 ? image_pitch : Wim;
-  if (pitch < Wim) return MGB_EINVAL;
-  const bool fast = itemsize >= 2 && (W * itemsize) % 16 == 0 && (pitch * itemsize) % 16 == 0 &&
-                    aligned16(tiles) && aligned16(image);
-  if (fast) {
-    const int u = itemsize / 2;  // 16-bit units per element
-    StitchParams p{};
-    p.tiles = (const uint16_t*)tiles; p.image = (uint16_t*)image;
-    p.CT = CT; p.T = (int)T; p.R = (int)R; p.Cc = (int)Cc;
-    p.H = (int)H; p.W = (int)(W * u); p.clip = clip * u; p.clip_y = clip; p.h = h; p.w = w * u;
-    p.Wim = pitch * u; p.Him = R * h; p.K = 1;
+  if (itemsize >= 2 && stitch_vectorisable(p)) {
     if (host_used_fast) *host_used_fast = 1;
     return run_stitch_fast<0>(p, st);
   }
-  const int64_t total = CT * R * h * Wim;
+  // the element-wise kernel takes the geometry in elements
+  const int We = p.W / u, w = p.w / u;
+  const int64_t pitch = p.Wim / u;
+  const int64_t total = p.CT * p.Him * p.Cc * w;
   const int g = grid_for(total);
   switch (itemsize) {
-    case 1: stitch_generic_kernel<uint8_t><<<g, kThreads, 0, st>>>((const uint8_t*)tiles, (uint8_t*)image, CT, (int)R, (int)Cc, (int)H, (int)W, clip, h, w, pitch); break;
-    case 2: stitch_generic_kernel<uint16_t><<<g, kThreads, 0, st>>>((const uint16_t*)tiles, (uint16_t*)image, CT, (int)R, (int)Cc, (int)H, (int)W, clip, h, w, pitch); break;
-    case 4: stitch_generic_kernel<uint32_t><<<g, kThreads, 0, st>>>((const uint32_t*)tiles, (uint32_t*)image, CT, (int)R, (int)Cc, (int)H, (int)W, clip, h, w, pitch); break;
-    default: stitch_generic_kernel<uint64_t><<<g, kThreads, 0, st>>>((const uint64_t*)tiles, (uint64_t*)image, CT, (int)R, (int)Cc, (int)H, (int)W, clip, h, w, pitch); break;
+    case 1: stitch_generic_kernel<uint8_t><<<g, kThreads, 0, st>>>((const uint8_t*)tiles, (uint8_t*)image, p.CT, p.R, p.Cc, p.H, We, p.clip_y, p.h, w, pitch); break;
+    case 2: stitch_generic_kernel<uint16_t><<<g, kThreads, 0, st>>>((const uint16_t*)tiles, (uint16_t*)image, p.CT, p.R, p.Cc, p.H, We, p.clip_y, p.h, w, pitch); break;
+    case 4: stitch_generic_kernel<uint32_t><<<g, kThreads, 0, st>>>((const uint32_t*)tiles, (uint32_t*)image, p.CT, p.R, p.Cc, p.H, We, p.clip_y, p.h, w, pitch); break;
+    default: stitch_generic_kernel<uint64_t><<<g, kThreads, 0, st>>>((const uint64_t*)tiles, (uint64_t*)image, p.CT, p.R, p.Cc, p.H, We, p.clip_y, p.h, w, pitch); break;
   }
   MGB_CUDA_LAUNCH_CHECK();
   return MGB_OK;
@@ -599,21 +600,13 @@ int mgb_flatfield_stitch_u16(const uint16_t* tiles, uint16_t* image, int64_t ima
                              int64_t T, int64_t R, int64_t Cc, int64_t H, int64_t W, int64_t overlap, int K,
                              const double* flat, const double* dark, const double* gain,
                              const double* bias, const double* maxima, void* stream) {
-  if (C < 0 || T < 0 || R < 0 || Cc < 0 || H <= 0 || W <= 0) return MGB_EINVAL;
-  if (overlap < 0 || overlap >= H || overlap >= W) return MGB_EINVAL;
   if (K != 1 && K != C) return MGB_EINVAL;
-  if (C * T == 0 || R == 0 || Cc == 0) return MGB_OK;
-  if (!tiles || !image || !flat || !dark || !gain || !bias || !maxima) return MGB_EINVAL;
-  if (H > INT32_MAX / 8 || W > INT32_MAX / 8 || R > INT32_MAX || Cc > INT32_MAX || K > 65535) return MGB_EUNSUPPORTED;
-  const int w = (int)(W - overlap), h = (int)(H - overlap);
-  const int64_t Wim = Cc * w;
-  const int64_t pitch = image_pitch > 0 ? image_pitch : Wim;
-  if (pitch < Wim) return MGB_EINVAL;
-  if (W % 8 != 0 || pitch % 8 != 0 || !aligned16(tiles) || !aligned16(image)) return MGB_EALIGN;
-  StitchParams p{};
-  p.tiles = tiles; p.image = image; p.CT = C * T; p.T = (int)T; p.R = (int)R; p.Cc = (int)Cc;
-  p.H = (int)H; p.W = (int)W; p.clip = (int)(overlap / 2); p.clip_y = p.clip; p.h = h; p.w = w;
-  p.Wim = pitch; p.Him = R * h; p.K = K;
+  const bool tables_ok = flat && dark && gain && bias && maxima;
+  StitchParams p;
+  const int rc = stitch_setup(tiles, image, image_pitch, C, T, R, Cc, H, W, overlap, 1, K, tables_ok,
+                              /*limits_first=*/false, &p);
+  if (rc != MGB_OK || p.CT == 0) return rc;
+  if (!stitch_vectorisable(p)) return MGB_EALIGN;
   p.gain = gain; p.bias = bias; p.flat = flat; p.dark = dark; p.maxima = maxima;
   return run_stitch_fast<1>(p, (cudaStream_t)stream);
 }

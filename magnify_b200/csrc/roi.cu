@@ -72,15 +72,14 @@ __device__ __forceinline__ uint64_t block_sum_u64(uint64_t v, uint64_t* smem) {
 
 // The median columns are left NaN: the caller fills them (roi_median kernels) when it wants them.
 __device__ __forceinline__ void write_record(double* o, uint64_t na, uint64_t nb, uint64_t a, uint64_t b) {
-  const double nan = __longlong_as_double(0x7ff8000000000000LL);
   o[0] = (double)na;
   o[1] = (double)nb;
   o[2] = (double)a;
   o[3] = (double)b;
   o[4] = (double)a / (double)na;   // 0/0 -> NaN, like nanmean over an empty mask
   o[5] = (double)b / (double)nb;
-  o[6] = nan;
-  o[7] = nan;
+  o[6] = nan_f64();
+  o[7] = nan_f64();
 }
 
 // Word path: 2 x 16-bit units per thread step (Lu even).  ALIGNED: source words 4-byte aligned.
@@ -251,7 +250,7 @@ roi_median_kernel(const TPix* __restrict__ roi, int64_t C, int64_t T, int L,
   };
   const uint32_t nvalid = block_count(cnt);
   if (nvalid == 0) {
-    if (threadIdx.x == 0) median[n * stride] = __longlong_as_double(0x7ff8000000000000LL);
+    if (threadIdx.x == 0) median[n * stride] = nan_f64();
     return;
   }
   const uint32_t k1 = (nvalid - 1) >> 1;  // lower middle (0-based)
@@ -342,7 +341,7 @@ roi_median_big_kernel(const TPix* __restrict__ roi, int64_t C, int64_t T, int L,
   uint32_t nvalid, above, lo;
   sweep(0xfffffffeu, &nvalid, &above, &lo);     // every valid key is <= 0xfffffffe
   if (nvalid == 0) {
-    if (threadIdx.x == 0) median[n * stride] = __longlong_as_double(0x7ff8000000000000LL);
+    if (threadIdx.x == 0) median[n * stride] = nan_f64();
     return;
   }
   const uint32_t k1 = (nvalid - 1) >> 1;
@@ -396,7 +395,7 @@ roi_stats_f32_kernel(const float* __restrict__ roi, int64_t C, int64_t T, int L,
     out[0] = s[0]; out[1] = s[1]; out[2] = s[2]; out[3] = s[3];
     out[4] = s[2] / s[0];   // 0 / 0 = NaN for an empty mask, like np.nanmean
     out[5] = s[3] / s[1];
-    out[6] = out[7] = __longlong_as_double(0x7ff8000000000000LL);   // medians: filled by the median kernel
+    out[6] = out[7] = nan_f64();   // medians: filled by the median kernel
   }
 }
 

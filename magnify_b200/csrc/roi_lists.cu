@@ -48,7 +48,6 @@ __device__ __forceinline__ void stage_mask(const uint8_t* __restrict__ g, int n,
     for (int i = tid; i < n; i += nth) s[i] = g[i];
   }
 }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 // generic-proxy accesses to shared memory before this, async-proxy (TMA) writes to it after
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 

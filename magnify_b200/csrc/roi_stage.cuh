@@ -79,19 +79,6 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map
       : "memory");
 }
 
-// 8 consecutive 16-bit units starting S units into the 16 units of (a, b).
-template <int S>
-__device__ __forceinline__ uint4 shift_units(const uint4& a, const uint4& b) {
-  const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
-  constexpr int o = S >> 1;
-  if constexpr ((S & 1) == 0) {
-    return make_uint4(w[o], w[o + 1], w[o + 2], w[o + 3]);
-  } else {
-    return make_uint4(__funnelshift_r(w[o], w[o + 1], 16), __funnelshift_r(w[o + 1], w[o + 2], 16),
-                      __funnelshift_r(w[o + 2], w[o + 3], 16), __funnelshift_r(w[o + 3], w[o + 4], 16));
-  }
-}
-
 // The timepoints whose mask timestep is tm (all of them when !MASKED), listed in tlist by one warp;
 // returns their number.
 template <bool MASKED>
@@ -128,7 +115,6 @@ __device__ __forceinline__ void load_window(const CUtensorMap* tmap, const TmaGa
 // the kernel does not compute them).  With peers, the 64-byte record goes straight into this rank's
 // block of the gathered buffer of EVERY rank (NVLink peer stores, one lane per peer): the
 // per-marker summaries are all-gathered by the kernel that computes them, no separate collective.
-__device__ __forceinline__ double nan_f64() { return __longlong_as_double(0x7ff8000000000000LL); }
 __device__ __forceinline__ void write_stats(const TmaGatherParams& p, int lane, int64_t n, double cf, double cb,
                                             double sf, double sb, double mf, double mb) {
   // called by the whole warp (all lanes hold the reduced values): lane 0 writes the local record,
@@ -241,11 +227,6 @@ __device__ __forceinline__ void consume_generic(const TmaGatherParams& p, const 
   *sf_out = sf;
   *sb_out = sb;
 }
-
-__device__ __forceinline__ void cp_async16_cg(uint32_t smem_addr, const void* gptr) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
-}
-
 
 template <int PAR>
 __device__ __forceinline__ uint32_t load_pair(const uint32_t* s32, uint32_t unit_off) {

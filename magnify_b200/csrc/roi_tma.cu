@@ -138,7 +138,7 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
     int row = lane / cpr, col = lane - row * cpr;
     const int drow = 32 / cpr, dcol = 32 - drow * cpr;
     for (int j = lane; j < n_chunks; j += 32) {
-      if (col <= lim) cp_async16_cg(dst0 + j * 16, base + (int64_t)row * p.Wu + col * 8);
+      if (col <= lim) cp_async16(dst0 + j * 16, base + (int64_t)row * p.Wu + col * 8);
       row += drow;
       col += dcol;
       if (col >= cpr) { col -= cpr; ++row; }
@@ -154,7 +154,7 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
     for (int s = 0; s < p.n_stages - 1; ++s) {
       const int i = warp + s * nw;
       if (i < n_items) issue_lsu(i, s);
-      asm volatile("cp.async.commit_group;" ::: "memory");
+      cp_async_commit();
     }
   }
   int s = 0;
@@ -169,7 +169,7 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
         if (nxt < n_items) issue_tma(nxt, rs);
       } else {
         if (nxt < n_items) issue_lsu(nxt, rs);
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
       }
     }
     int64_t c, t;
@@ -183,9 +183,9 @@ roi_gather_tma_kernel(const __grid_constant__ CUtensorMap tmap, const TmaGatherP
     } else {
       // all but the newest n_stages-1 groups are complete -> this item's chunks have landed
       switch (p.n_stages) {
-        case 2: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
-        case 3: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
-        default: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
+        case 2: cp_async_wait<1>(); break;
+        case 3: cp_async_wait<2>(); break;
+        default: cp_async_wait<3>(); break;
       }
       __syncwarp();
     }

@@ -213,29 +213,37 @@ class FlatFieldPlan:
         return self._workspace
 
 
+def _maxima_pass(block: torch.Tensor, channels: int, planes: int, flat: torch.Tensor, dark: torch.Tensor, k: int,
+                 plan: FlatFieldPlan) -> None:
+    """Pass 1 over a contiguous `block` of `channels` x `planes` planes of (H, W) (its trailing dims)
+    against k flat/dark tables of (H, W) (k == 1: one for every channel), max-accumulated into
+    plan.maxima."""
+    hw = block.shape[-2] * block.shape[-1]
+    if block.dtype == torch.uint16 and hw % 8 == 0 and block.data_ptr() % 16 == 0:
+        base = -(-(hw // 8) // 256) * k
+        n_planes = channels * planes if k == 1 else planes
+        splits = max(1, min(n_planes // 8 if n_planes >= 16 else 1, -(-sm_count() * 16 // base), 4096))
+        ws = plan.workspace(splits * k * hw * 2, block.device)
+        _lib.call("mgb_flatfield_tilemax_u16", _ptr(block), channels, planes, hw, k, splits, _ptr(ws), _stream())
+        _lib.call("mgb_flatfield_maxima", _ptr(ws), splits, k, hw, _ptr(flat), _ptr(dark), _ptr(plan.maxima),
+                  _stream())
+    else:
+        if block.dtype not in _DTYPE_CODE:
+            raise TypeError(f"flat-field supports uint8/uint16/float32/float64 tiles, got {block.dtype}")
+        _lib.call("mgb_flatfield_maxima_generic", _ptr(block), _DTYPE_CODE[block.dtype], channels, planes, hw, k,
+                  _ptr(flat), _ptr(dark), _ptr(plan.maxima), _stream())
+
+
 def flatfield_maxima(tiles: torch.Tensor, plan: FlatFieldPlan) -> torch.Tensor:
     """Pass 1: the two global maxima (M, M2) of preprocess.py:84,86 over this rank's tiles, as a
     float64[2] device tensor (plan.maxima).  Multi-GPU callers all-reduce it with MAX."""
     _check(tiles, "tiles", ndim=6)
-    c, t, r, cc, h, w = tiles.shape
-    planes, hw = t * r * cc, h * w
+    c, t, r, cc = tiles.shape[:4]
     with torch.cuda.device(tiles.device):
         plan.maxima.zero_()
         if tiles.numel() == 0:
             return plan.maxima
-        if tiles.dtype == torch.uint16 and hw % 8 == 0 and tiles.data_ptr() % 16 == 0:
-            base = -(-(hw // 8) // 256) * plan.k
-            n_planes = c * planes if plan.k == 1 else planes
-            splits = max(1, min(n_planes // 8 if n_planes >= 16 else 1, -(-sm_count() * 16 // base), 4096))
-            ws = plan.workspace(splits * plan.k * hw * 2, tiles.device)
-            _lib.call("mgb_flatfield_tilemax_u16", _ptr(tiles), c, planes, hw, plan.k, splits, _ptr(ws), _stream())
-            _lib.call("mgb_flatfield_maxima", _ptr(ws), splits, plan.k, hw, _ptr(plan.flat), _ptr(plan.dark),
-                      _ptr(plan.maxima), _stream())
-        else:
-            if tiles.dtype not in _DTYPE_CODE:
-                raise TypeError(f"flat-field supports uint8/uint16/float32/float64 tiles, got {tiles.dtype}")
-            _lib.call("mgb_flatfield_maxima_generic", _ptr(tiles), _DTYPE_CODE[tiles.dtype], c, planes, hw, plan.k,
-                      _ptr(plan.flat), _ptr(plan.dark), _ptr(plan.maxima), _stream())
+        _maxima_pass(tiles, c, t * r * cc, plan.flat, plan.dark, plan.k, plan)
     return plan.maxima
 
 
@@ -253,18 +261,7 @@ def flatfield_maxima_accumulate(block: torch.Tensor, plan: FlatFieldPlan, channe
     flat = plan.flat.view(-1)[k_off:k_off + hw]
     dark = plan.dark.view(-1)[k_off:k_off + hw]
     with torch.cuda.device(block.device):
-        if block.dtype == torch.uint16 and hw % 8 == 0 and block.data_ptr() % 16 == 0:
-            base = -(-(hw // 8) // 256)
-            splits = max(1, min(planes // 8 if planes >= 16 else 1, -(-sm_count() * 16 // base), 4096))
-            ws = plan.workspace(splits * hw * 2, block.device)
-            _lib.call("mgb_flatfield_tilemax_u16", _ptr(block), 1, planes, hw, 1, splits, _ptr(ws), _stream())
-            _lib.call("mgb_flatfield_maxima", _ptr(ws), splits, 1, hw, _ptr(flat), _ptr(dark), _ptr(plan.maxima),
-                      _stream())
-        else:
-            if block.dtype not in _DTYPE_CODE:
-                raise TypeError(f"flat-field supports uint8/uint16/float32/float64 tiles, got {block.dtype}")
-            _lib.call("mgb_flatfield_maxima_generic", _ptr(block), _DTYPE_CODE[block.dtype], 1, planes, hw, 1,
-                      _ptr(flat), _ptr(dark), _ptr(plan.maxima), _stream())
+        _maxima_pass(block, 1, planes, flat, dark, 1, plan)
 
 
 def flatfield_stitch(
@@ -336,10 +333,8 @@ def flatfield_correct(tiles: torch.Tensor, flatfield=1.0, darkfield=0.0, plan=No
         return tiles.clone()
     # Every tile is its own 1x1 "image": same kernel, overlap 0.
     as_images = tiles.view(c, t * r * cc, 1, 1, h, w)
-    plan_shape = plan.tile_shape
     dense = torch.empty((c, t * r * cc, h, w), dtype=tiles.dtype, device=tiles.device)   # tile layout is dense
     out = flatfield_stitch(as_images, overlap=0, plan=plan, maxima=maxima, group=group, out=dense)
-    plan.tile_shape = plan_shape
     return out.view(tiles.shape)
 
 

@@ -59,14 +59,41 @@ def test_disc_halfwidths_host_entry_point(lib, golden):
 
 
 def test_argument_errors_before_any_launch(lib):
-    """Validation happens on the host: these return MGB_EINVAL without touching a GPU."""
+    """Validation happens on the host: these return a status without touching a GPU."""
     import ctypes
 
     p = ctypes.c_void_p(0)
+    q16 = ctypes.c_void_p(4096)   # non-null and 16-byte aligned; never dereferenced, every call returns first
     assert lib.mgb_stitch(p, p, 0, 1, 1, 2, 2, 50, 50, -5, 2, None, p) == -1     # stitch.py:8-9
     assert lib.mgb_stitch(p, p, 0, 1, 1, 2, 2, 50, 50, 100, 2, None, p) == -1    # stitch.py:16-20
     assert lib.mgb_stitch(p, p, 0, 1, 1, 2, 2, 50, 50, 4, 3, None, p) == -1      # itemsize
     assert lib.mgb_stitch(p, p, 0, 0, 1, 2, 2, 50, 50, 4, 2, None, p) == 0       # empty: nothing to do
+    assert lib.mgb_stitch(q16, q16, 10, 1, 1, 2, 2, 50, 56, 4, 2, None, p) == -1  # pitch < Cc * (W - overlap)
+
+    ff = lib.mgb_flatfield_stitch_u16
+    assert ff(p, p, 0, 1, 1, 2, 2, 50, 56, -5, 1, *[p] * 6) == -1                 # stitch.py:8-9
+    assert ff(p, p, 0, 1, 1, 2, 2, 50, 56, 50, 1, *[p] * 6) == -1                 # stitch.py:16-20
+    assert ff(p, p, 0, 0, 1, 2, 2, 50, 56, 4, 2, *[p] * 6) == -1                  # K neither 1 nor C
+    assert ff(p, p, 0, 0, 1, 2, 2, 50, 56, 4, 1, *[p] * 6) == 0                   # empty: nothing to do
+    assert ff(q16, q16, 0, 1, 1, 2, 2, 50, 56, 4, 1, *[q16] * 4, p, p) == -1      # null maxima table
+    assert ff(q16, q16, 10, 1, 1, 2, 2, 50, 56, 4, 1, *[q16] * 6) == -1           # pitch < Cc * (W - overlap)
+    assert ff(q16, q16, 0, 1, 1, 2, 2, 50, 52, 4, 1, *[q16] * 6) == -2            # W not whole 16-byte vectors
+
+    # Size limits: mgb_stitch checks them before the empty-stack shortcut and the null pointers,
+    # mgb_flatfield_stitch_u16 after them.
+    tall = (2**31 - 1) // 8 + 1
+    assert lib.mgb_stitch(p, p, 0, 0, 1, 2, 2, tall, 56, 4, 2, None, p) == -3
+    assert ff(p, p, 0, 0, 1, 2, 2, tall, 56, 4, 1, *[p] * 6) == 0
+    assert lib.mgb_stitch(p, p, 0, 1, 1, 2, 2, tall, 56, 4, 2, None, p) == -3
+    assert ff(p, p, 0, 1, 1, 2, 2, tall, 56, 4, 1, *[p] * 6) == -1
+    assert lib.mgb_stitch(q16, q16, 0, 1, 1, 2, 2, tall, 56, 4, 2, None, p) == -3
+    assert ff(q16, q16, 0, 1, 1, 2, 2, tall, 56, 4, 1, *[q16] * 6) == -3
+    assert lib.mgb_stitch(p, p, 0, 1, 1, 2**31, 0, 50, 56, 4, 2, None, p) == -3  # R > INT32_MAX, no tile columns
+    assert ff(p, p, 0, 1, 1, 2**31, 0, 50, 56, 4, 1, *[p] * 6) == 0
+    assert ff(p, p, 0, 70000, 0, 2, 2, 50, 56, 4, 70000, *[p] * 6) == 0           # K > 65535 tables
+    assert ff(p, p, 0, 70000, 1, 2, 2, 50, 56, 4, 70000, *[p] * 6) == -1
+    assert ff(q16, q16, 0, 70000, 1, 2, 2, 50, 56, 4, 70000, *[q16] * 6) == -3
+
     assert lib.mgb_bounding_boxes(p, p, 4, 72, 50, 50, p, p, p) == -1         # image smaller than box
     assert lib.mgb_roi_gather(p, 0, 1, 1, 100, 100, 2, p, p, 0, 72, p, p) == 0  # zero markers
     assert lib.mgb_chip_masks(p, p, 15, 30, 0, 72, p, p, p, p) == 0

@@ -473,7 +473,7 @@ def test_flatfield_exact_pixel_in_fast_vector(cuda_device, stitch_variant, col):
 
 # -------------------------------------------------------------------------- maxima, pass 1
 def tilemax_splits(n_planes, hw, K, sm_count):
-    """The split of the uint16 maxima pass over planes (ops.flatfield_maxima restated)."""
+    """The split of the uint16 maxima pass over planes (ops._maxima_pass restated)."""
     base = -(-(hw // 8) // 256) * K
     return max(1, min(n_planes // 8 if n_planes >= 16 else 1, -(-sm_count * 16 // base), 4096))
 
